@@ -17,7 +17,10 @@ being benchmarked and compares x_t, C and the replicated state with the CPU orac
 numpy oracle) run by rank 0 on the global problem; the result goes into the JSON line (`parity`) and a relative error
 above the tolerance (1e-9 fp64, 1e-4 fp32) ends the run with exit code 3 before any number is printed as valid.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W]                    # CUDA arm
+--dump-outputs DIR writes, after the timed steps, what the last timed step computed (see dump_outputs); the inputs are
+generated from a fixed seed, so two builds run with the same arguments can be compared output for output.
+
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]  # CUDA arm
   python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]   # reference arm: CPU oracle port on the host cores
   python bench.py --impl nccl --gpus N ...                               # baseline: one launch per step + ncclAllReduce
 """
@@ -68,7 +71,13 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-steps", type=int, default=0, help="filter steps of the CPU baseline sample (0 = auto)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (X, and the filter state) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm (--impl b200)")
     if a.workload == "L":
         a.d, a.r, a.T = a.d or 1_000_000, a.r or 16, a.T or 10_000
     else:
@@ -347,6 +356,32 @@ def traffic_for(d_loc, r, dtype, W):
         return None
 
 
+DUMP_FILE_BYTES = 8 << 20        # per .npy file of --dump-outputs; at most 8 files, so 64 MB in all
+DUMP_SEED = 12345
+
+
+def dump_outputs(ctx, arrays):
+    """--dump-outputs: write `arrays` -- name -> (local, off, total) -- as DIR/<name>.npy from rank 0.  `local` holds rows
+    [off, off + len(local)) of a (total, ...) array whose rows are split over the ranks; total = None marks an array that
+    every rank holds whole.  An array larger than DUMP_FILE_BYTES is written as a fixed, seeded sample of its rows
+    (sorted row indices), so two runs with the same arguments write the same rows.  Every rank must call this."""
+    torch = ctx["torch"]
+    for name, (local, off, total) in arrays.items():
+        sharded = total is not None
+        total = total if sharded else local.shape[0]
+        row_bytes = local[:1].numel() * local.element_size()
+        k = max(1, DUMP_FILE_BYTES // row_bytes)
+        idx = torch.arange(total) if total <= k else torch.from_numpy(np.sort(np.random.default_rng(DUMP_SEED).choice(total, k, replace=False)))
+        mine = (idx >= off) & (idx < off + local.shape[0])
+        out = torch.zeros((len(idx),) + tuple(local.shape[1:]), dtype=local.dtype, device=local.device)
+        out[mine.to(local.device)] = local[(idx[mine] - off).to(local.device)]
+        if sharded and ctx["world"] > 1:
+            ctx["dist"].all_reduce(out)          # every row has one owner and zeros elsewhere: the sum is exact
+        if ctx["rank"] == 0:
+            os.makedirs(ctx["args"].dump_outputs, exist_ok=True)
+            np.save(os.path.join(ctx["args"].dump_outputs, name + ".npy"), out.cpu().numpy())
+
+
 # --------------------------------------------------------------------------------------------------
 # workload L
 # --------------------------------------------------------------------------------------------------
@@ -466,6 +501,12 @@ def run_workload_L(ctx):
     filter_steps = args.steps * W
     value = filter_steps / (total_ms * 1e-3)
     info = eng.launch_info()
+    if args.dump_outputs:
+        # X of the last launch (W, r) and the state it leaves: C row-sharded, the rest replicated (leading dim: 1 series)
+        st = eng.get_state()
+        arrays = {"X": (Xbuf[0], 0, None), "C": (st["C"], row0, d)}
+        arrays.update({k: (st[k].unsqueeze(0), 0, None) for k in ("x", "P", "V", "Q", "rho", "lam")})
+        dump_outputs(ctx, arrays)
 
     # ---- roofline of the dominant (only) kernel, against the bound of ITS regime (SURVEY.md 8(d)) ----
     peaks = _peaks()
@@ -641,6 +682,12 @@ def run_workload_B(ctx):
     per_launch_ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]
     value = args.steps * W * S / (total_ms * 1e-3)
     info = eng.launch_info()
+    if args.dump_outputs:
+        # the timed launches return no X: the state they leave, series-sharded (C as rows of (series, row) pairs)
+        st = {k: (v.unsqueeze(0) if S_loc == 1 else v) for k, v in eng.get_state().items() if v is not None}
+        arrays = {"C": (st["C"].reshape(S_loc * d, r), s0 * d, S * d)}
+        arrays.update({k: (st[k], s0, S) for k in ("x", "P", "V", "Q", "rho", "lam")})
+        dump_outputs(ctx, arrays)
     peaks = _peaks()
     mean_launch_s = float(np.mean(per_launch_ms)) * 1e-3
     clk = (clocks.get("sm_mhz") or peaks.get("sm_max_mhz") or 1965.0) * 1e6

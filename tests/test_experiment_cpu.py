@@ -61,8 +61,8 @@ def test_argument_checks():
 def test_published_pinning_summary():
     """tests/golden/pin_published.py replayed all 18 published result files whose input CSVs ship with the
     reference (3 datasets x 3 percentages x 2 methods): inputs of all 100 repeats by hash, results of the first
-    repeats through the oracle.  The summary it wrote is committed; where the reference is present, one file is
-    replayed live."""
+    repeats through the oracle.  The summary it wrote is committed; one file (PM2.5, 20 %, PSMF) is replayed here
+    from the stored data set (LondonAir_PM25.csv, kept in impute_pm25_30.npz) against its stored published results."""
     import json
     import os
     here = os.path.dirname(os.path.abspath(__file__))
@@ -72,10 +72,8 @@ def test_published_pinning_summary():
     # end-of-fit scalars of the d x d reference against the O(d r^2) oracle: 17 files <= 1.3e-11, sp500 40 % rPSMF 1.25e-9
     assert s["max_rel_err_error_predict"] < 2e-9 and s["max_rel_err_error_full"] < 2e-9
     assert s["max_abs_err_inside_sig"] == 0.0
-    ref = "/root/reference/ExperimentImpute"
-    if os.path.exists(os.path.join(ref, "data", "LondonAir_PM25.csv")):
-        pub = json.load(open(os.path.join(ref, "output", "LondonAir_PM25_20_PSMF.json")))
-        Yorig = np.genfromtxt(os.path.join(ref, "data", "LondonAir_PM25.csv"), delimiter=",")
-        out = ex.run_impute_experiment(Yorig, "PSMF", 20, seed=pub["seed"], repeats=1, fit=_oracle_fit(False))
-        assert out["hashes"]["Y"][0] == pub["hashes"]["Y"][0]
-        assert abs(out["results"]["error_full"][0] - pub["results"]["error_full"][0]) / pub["results"]["error_full"][0] < 1e-9
+    pub = json.load(open(os.path.join(here, "golden", "published_results.json")))["files"]["LondonAir_PM25_20_PSMF"]
+    Yorig = load_golden("impute_pm25_30")["Yorig"]
+    out = ex.run_impute_experiment(Yorig, "PSMF", 20, seed=pub["seed"], repeats=1, fit=_oracle_fit(False))
+    assert out["hashes"]["Y"][0] == pub["hashes"]["Y"][0]
+    assert abs(out["results"]["error_full"][0] - pub["results"]["error_full"][0]) / pub["results"]["error_full"][0] < 1e-9

@@ -236,3 +236,33 @@ def test_reference_arm_prints_the_config_record_of_the_cuda_arm():
     assert line["metric"] == bench.metric_name(args) and line["unit"] == bench.unit_name(args) and line["higher_is_better"] is True
     assert line["cpu_baseline"]["kind"] in ("port", "reference") and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["value"] == line["value"] > 0
+
+
+def test_bench_dump_outputs_is_bounded_and_reproducible(tmp_path):
+    """bench.py --dump-outputs: an array up to 8 MB is written whole, a larger one as the same seeded sample of its rows on
+    every run; the shard of a row-split array lands on its global rows; --steps must be >= 1."""
+    import os
+    import subprocess
+    import sys
+    import torch
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+
+    class Args:
+        pass
+    d, r = 300_000, 16                                                    # 38 MB of float64: sampled
+    C = torch.arange(d * r, dtype=torch.float64).reshape(d, r)
+    X = torch.randn(500, r, dtype=torch.float64)
+    for run in ("a", "b"):
+        a = Args()
+        a.dump_outputs = str(tmp_path / run)
+        ctx = dict(torch=torch, dist=None, world=1, rank=0, args=a)
+        bench.dump_outputs(ctx, {"X": (X, 0, None), "C": (C[1000:], 1000, d)})      # this rank holds rows 1000 .. d - 1
+    Xa, Ca, Cb = (np.load(str(tmp_path / p)) for p in ("a/X.npy", "a/C.npy", "b/C.npy"))
+    assert np.array_equal(Xa, X.numpy()) and np.array_equal(Ca, Cb)
+    assert Ca.nbytes <= bench.DUMP_FILE_BYTES and Ca.shape == (bench.DUMP_FILE_BYTES // (r * 8), r)
+    idx = np.sort(np.random.default_rng(bench.DUMP_SEED).choice(d, len(Ca), replace=False))
+    assert np.array_equal(Ca, np.where((idx >= 1000)[:, None], C.numpy()[idx], 0.0))         # other ranks' rows: zero here
+    bad = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "0"], capture_output=True, text=True, cwd=root)
+    assert bad.returncode == 2 and "--steps" in bad.stderr
