@@ -270,7 +270,9 @@ __device__ __forceinline__ void row_stats(TileAcc<R>& A, const Smem<R>& sh, doub
 #pragma unroll
     for (int j = 0; j < R; ++j) A.v[j] = fma(ew, c[j], A.v[j]);               // b = CM' Ri diff
     const double e2 = e * e;
-    A.v[R + 0] = fma(inb ? w : 0.0, e2, A.v[R + 0]);                           // diff' Ri diff
+    // diff' Ri diff.  A missing row with a zero residual adds nothing, also when a = 0 makes w0 = 1/a infinite (x'Vx
+    // vanishes exactly after a step with every row missing at r = 1): the same rule as s = w1 q1 + w0 q0 of the TMA kernel
+    A.v[R + 0] = fma((inb && (mi || e2 != 0.0)) ? w : 0.0, e2, A.v[R + 0]);
     A.v[R + 1] += mi ? e2 : 0.0;                                               // rPSMF.py:112-114 (observed rows)
     A.v[R + 2] += mi ? 0.0 : e2;                                               //                  (missing rows)
     A.v[R + 3] += mi ? 1.0 : 0.0;

@@ -22,27 +22,68 @@ def _torch():
     return torch
 
 
-def _engine_run(d, r, Y, M, C0, x0, init, robust, ctas=0, dtype=None, chunks=None, **kw):
+def _padded(a, dtype, dev, pad=0, gap=0, fill=0):
+    """(S, T, d) device view of host array `a` inside a larger buffer filled with `fill`: rows of d + pad elements and
+    `gap` more elements between series.  Returns (view, buffer)."""
+    torch = _torch()
+    S, T, d = a.shape
+    ld = d + pad
+    sst = T * ld + gap
+    buf = torch.full((S * sst,), fill, dtype=dtype, device=dev)
+    view = buf.as_strided((S, T, d), (sst, ld, 1))
+    view.copy_(torch.as_tensor(a).to(dtype))
+    return view, buf
+
+
+def _engine_run(d, r, Y, M, C0, x0, init, robust, ctas=0, dtype=None, chunks=None, S=None, pad=0, gap=0, rec_pad=0,
+                want_grad=False, Yorig=None, E=None, **kw):
+    """Run the engine over Y (T, d), or (S, T, d) with S series, in the launches given by `chunks`.  `pad` / `gap` put Y, M
+    (and Yorig, E) inside larger buffers (rows of d + pad elements, gaps between series); `rec_pad` writes Yrec into rows
+    of d + rec_pad elements whose padding is NaN and must stay so.  Returns (X, Yrec, scal, state, launch_info); with S
+    the arrays keep the series axis, the state holds the theta gradient ("grad", summed over the launches) when
+    `want_grad` and the fused evaluation sums ("eval") when E is given."""
     torch = _torch()
     from rpsmf_b200 import FilterEngine
     dtype = dtype or torch.float64
-    eng = FilterEngine(d, r, dtype=dtype, robust=robust, ctas=ctas, **kw)
-    eng.set_state(C_=C0, V=init["V"], P=init["P"], x=x0, Q=init["Q"], rho=[init["rho"]], lam=[init["lam"]],
+    eng = FilterEngine(d, r, dtype=dtype, robust=robust, ctas=ctas, n_series=S or 1, **kw)
+    eng.set_state(C_=C0, V=init["V"], P=init["P"], x=x0, Q=init["Q"], rho=np.atleast_1d(init["rho"]), lam=[init["lam"]],
                   theta=init.get("theta"))
     dev = eng.device
-    Yd = torch.as_tensor(Y, dtype=dtype).to(dev)
-    Md = None if M is None else torch.as_tensor(M).to(dev)
-    T = Y.shape[0]
+    one = S is None
+    Y3 = Y[None] if one else Y
+    Yd, _ = _padded(Y3, dtype, dev, pad, gap, float("nan"))
+    Md = None if M is None else _padded(M[None] if one else M, torch.uint8, dev, pad, gap, 1)[0]
+    Yod = None if Yorig is None else _padded(Yorig[None] if one else Yorig, dtype, dev, pad, gap, float("nan"))[0]
+    Ed = None if E is None else _padded(E[None] if one else E, torch.uint8, dev, pad, gap, 1)[0]
+    Sn, T = Y3.shape[0], Y3.shape[1]
+    Yrec, rec_buf = _padded(np.zeros((Sn, T, d)), dtype, dev, rec_pad, gap if rec_pad else 0, float("nan"))
     bounds = [0, T] if chunks is None else chunks
-    Xs, Yr, Sc = [], [], []
+    Xs, Sc, grad, ev = [], [], 0.0, 0.0
     for a, b in zip(bounds[:-1], bounds[1:]):
-        out = eng.run(Yd[a:b], None if Md is None else Md[a:b], k0=1 + a, want_X=True, want_Yrec=True, want_scal=True)
+        out = eng.run(Yd[:, a:b], None if Md is None else Md[:, a:b], k0=1 + a, want_X=True, Yrec_out=Yrec[:, a:b],
+                      want_scal=True, want_grad=want_grad, Yorig=None if Yod is None else Yod[:, a:b],
+                      E=None if Ed is None else Ed[:, a:b])
         assert eng.status() == -1
-        Xs.append(out["X"].cpu().numpy()); Yr.append(out["Yrec"].double().cpu().numpy()); Sc.append(out["scal"].cpu().numpy())
+        Xs.append(out["X"].reshape(Sn, b - a, r).cpu().numpy()); Sc.append(out["scal"].reshape(Sn, b - a, -1).cpu().numpy())
+        if want_grad:
+            grad = grad + out["grad"].cpu().numpy()
+        if E is not None:
+            ev = ev + out["eval"].cpu().numpy()
     st = {k: (v.double().cpu().numpy() if v is not None else None) for k, v in eng.get_state().items()}
+    if want_grad:
+        st["grad"] = grad
+    if E is not None:
+        st["eval"] = ev
     info = eng.launch_info()
     eng.close()
-    return np.concatenate(Xs), np.concatenate(Yr), np.concatenate(Sc), st, info
+    # the rows of Yrec were written, nothing around them
+    keep = torch.ones_like(rec_buf, dtype=torch.bool)
+    keep.as_strided(Yrec.shape, Yrec.stride()).fill_(False)
+    assert bool(rec_buf[keep].isnan().all())
+    X, Yr, Sc = np.concatenate(Xs, axis=1), Yrec.double().cpu().numpy(), np.concatenate(Sc, axis=1)
+    if one:
+        X, Yr, Sc = X[0], Yr[0], Sc[0]
+    return X, Yr, Sc, st, info
 
 
 def _oracle_run(Y, M, C0, x0, init, cfg, k0=1):
