@@ -56,6 +56,11 @@ typedef struct psmf_engine* psmf_handle;
 #define PSMF_RHO_VECTOR   128  /* R is diagonal but NOT uniform (psmf.py:144-152 takes the Woodbury branch for any diagonal R; the
                                * flat functions accept any (d, d) R): `rho` of psmf_set_state / psmf_get_state is then
                                * (n_series, d) = diag(R).  One GPU, direct-load kernel.                                */
+#define PSMF_GRAD_LINEAR  256  /* PSMF_DYN_LINEAR only: grad_out is the gradient of the summed incremental log-likelihood with
+                               * respect to A and c (x_bar = A x + c, N, eta and V held fixed, as for the cos gradient):
+                               * [G_A = sum_k gf_k x_{k-1}' (r x r row-major) | G_c = sum_k gf_k (r)] per series, gf_k =
+                               * d ell_k / d x_bar_k.  d ell / d theta = <dA/dtheta, G_A>_F + <dc/dtheta, G_c> for any A(theta),
+                               * c(theta): the caller closes the chain rule.  All kernels; row-sharded ranks agree bit for bit */
 
 /* dynamics f_theta(x, k) of the predict half (psmf.py:104-115) */
 #define PSMF_DYN_IDENTITY 0    /* RandomWalk, nonlinearities.py:42-56; Impute scripts */
@@ -135,7 +140,8 @@ typedef struct psmf_io {
     const double*  xbar_ext;   /* PSMF_DYN_EXTERNAL: (n_series, r)                                    */
     const double*  F_ext;      /* PSMF_DYN_EXTERNAL: (n_series, r, r) row-major                       */
     double*        grad_out;   /* (n_series, r) sum over the run of d ell_k / d theta (PSMF_DYN_COS), or NULL
-                                * (_store_gradient, psmf.py:167-177); PSMF_DYN_EXTERNAL: d ell_k / d f of the one step */
+                                * (_store_gradient, psmf.py:167-177); PSMF_DYN_EXTERNAL: d ell_k / d f of the one step;
+                                * PSMF_GRAD_LINEAR: (n_series, r*r + r) [G_A row-major | G_c] summed over this run       */
     /* fused evaluation (all NULL / 0 = off): RMSE of the one-step predictions over the entries marked in E and the
      * number of original values inside the sig-sigma interval, accumulated in the row pass -- no (n, d) Yrec /
      * YrecL / YrecH arrays (rPSMF.py:67-69,121-123,139; common.py:79-94).  Direct-load and batch kernels only. */

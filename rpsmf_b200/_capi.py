@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("PSMF_B200_LIB") or os.path.join(_HERE, "libpsmf_b200.so")   # the override is for kernel experiments
 
 F64, F32 = 0, 1
-ROBUST, SIMPLIFIED, CUPDATE_VT, FIXED_LAMBDA, LL_STUDENT, NAN_MASK, RHO_VECTOR = 1, 2, 4, 16, 32, 64, 128
+ROBUST, SIMPLIFIED, CUPDATE_VT, FIXED_LAMBDA, LL_STUDENT, NAN_MASK, RHO_VECTOR, GRAD_LINEAR = 1, 2, 4, 16, 32, 64, 128, 256
 DYN_IDENTITY, DYN_COS, DYN_LINEAR, DYN_EXTERNAL = 0, 1, 2, 3
 KERNEL_AUTO, KERNEL_DIRECT, KERNEL_STREAM, KERNEL_BATCH = 0, 1, 2, 3
 XCHG_NVLINK, XCHG_EXTERNAL = 0, 1

@@ -219,6 +219,8 @@ extern "C" int psmf_create(psmf_handle* out, const psmf_config* cfg) {
     if ((cfg->flags & PSMF_RHO_VECTOR) && (cfg->world_size > 1 || cfg->kernel == 2 || cfg->kernel == 3))
         return fail(nullptr, PSMF_E_INVALID, "PSMF_RHO_VECTOR (non-uniform diagonal R) runs on the direct-load kernel of one GPU: "
                                              "world_size 1, kernel AUTO or DIRECT");
+    if ((cfg->flags & PSMF_GRAD_LINEAR) && cfg->dynamics != PSMF_DYN_LINEAR)
+        return fail(nullptr, PSMF_E_INVALID, "PSMF_GRAD_LINEAR is the gradient with respect to A and c: it needs PSMF_DYN_LINEAR");
     if (cfg->exchange == PSMF_XCHG_EXTERNAL && cfg->n_series > 1)
         return fail(nullptr, PSMF_E_INVALID, "PSMF_XCHG_EXTERNAL shards ONE series by rows (n_series must be 1)");
     if (cfg->world_size < 1 || cfg->world_size > PSMF_MAX_PEERS || cfg->rank < 0 || cfg->rank >= cfg->world_size)
@@ -542,13 +544,20 @@ static int run_impl(psmf_handle h, const psmf_io* io, int64_t n_steps, int64_t k
     bool use3 = h->batch_ok && !external &&
                 (h->cfg.kernel == 3 || (h->cfg.kernel == 0 && h->cfg.ctas <= 0 && (h->S > 1 || h->ntiles <= 32)));
     size_t dyn3 = h->dyn_smem3;
-    if (use3 && eval) {
-        dyn3 = batch_dyn(h->ntiles, h->R, h->esize, true);
+    // PSMF_GRAD_LINEAR: the accumulator G_A (R * R doubles) goes behind the other dynamic shared memory of the direct-load and
+    // batch kernels; the TMA-staged control CTA keeps it in its own dynamic shared memory, which is at least one chunk slot
+    // (>= 512 R bytes > 8 R^2)
+    const size_t glin = (h->cfg.flags & PSMF_GRAD_LINEAR) ? (size_t)h->R * h->R * sizeof(double) : 0;
+    if (use3 && (eval || glin)) {
+        dyn3 = batch_dyn(h->ntiles, h->R, h->esize, eval);
+        p.glin_off = (int64_t)dyn3;
+        dyn3 += glin;
         LaunchShape sb;
         if (dyn3 > (size_t)h->maxsmem ||
             (h->batch_nw8 ? SHAPE_B8 : SHAPE_B4)[h->R](h->cfg.dtype, dyn3, &sb) != cudaSuccess || sb.max_ctas_per_sm < 1) {
             cudaGetLastError();
-            if (h->cfg.kernel == 3) return fail(h, PSMF_E_NOMEM, "batch kernel: no shared memory left for the evaluation buffers");
+            if (h->cfg.kernel == 3)
+                return fail(h, PSMF_E_NOMEM, "batch kernel: no shared memory left for the evaluation buffers / the gradient accumulator");
             use3 = false;
         }
     }
@@ -579,6 +588,7 @@ static int run_impl(psmf_handle h, const psmf_io* io, int64_t n_steps, int64_t k
     } else if (use2) {
         p.cps = h->cps2;
         p.nslot = h->nslot;
+        p.glin_off = 0;                   // G_A at the start of the control CTA's dynamic shared memory
         p.trace_cta = h->cps2;
         // streaming from HBM: 12 of the 14 pass warps (3 per scheduler; a multiple of the 4 tiles of a chunk) keep up
         // with the ring and leave issue slots to the producer -- measured optimum at r = 16 under the power cap;
@@ -594,14 +604,16 @@ static int run_impl(psmf_handle h, const psmf_io* io, int64_t n_steps, int64_t k
         h->last_dyn = h->dyn_smem2;
     } else {
         size_t dyn1 = h->dyn_smem;
-        if (eval) {
+        if (eval || glin) {
             const int64_t tiles_per = (h->ntiles + h->cps - 1) / h->cps + 1;
-            dyn1 += (size_t)tiles_per * TILE * 17 + 16;
+            if (eval) dyn1 += (size_t)tiles_per * TILE * 17 + 16;
+            p.glin_off = (int64_t)dyn1;
+            dyn1 += glin;
             LaunchShape sh1;
             if (((h->cfg.flags & PSMF_RHO_VECTOR) ? SHAPE_V : SHAPE)[h->R](h->cfg.dtype, dyn1, &sh1) != cudaSuccess || sh1.max_ctas_per_sm < 1 ||
                 (h->cooperative && h->cps > h->num_sms * sh1.max_ctas_per_sm)) {
                 cudaGetLastError();
-                return fail(h, PSMF_E_NOMEM, "no shared memory left for the evaluation buffers at this d / grid");
+                return fail(h, PSMF_E_NOMEM, "no shared memory left for the evaluation buffers / the gradient accumulator at this d / grid");
             }
         }
         CK(h, ((h->cfg.flags & PSMF_RHO_VECTOR) ? LAUNCH_V : LAUNCH)[h->R](p, h->cfg.dtype, h->S * h->cps, dyn1, st, h->cooperative));

@@ -21,7 +21,7 @@ constexpr int MAX_PEERS = 8;
 
 // flags (mirror include/psmf_b200.h)
 constexpr int F_ROBUST = 1, F_SIMPLIFIED = 2, F_CUPDATE_VT = 4, F_FIXED_LAMBDA = 16, F_LL_STUDENT = 32, F_NAN_MASK = 64,
-              F_RHO_VECTOR = 128;
+              F_RHO_VECTOR = 128, F_GRAD_LINEAR = 256;
 constexpr int DYN_IDENTITY = 0, DYN_COS = 1, DYN_LINEAR = 2, DYN_EXTERNAL = 3;
 constexpr int NEVAL = 4;     // fused evaluation record (include/psmf_b200.h PSMF_EVAL_*)
 // debug-only flag bits (env PSMF_DEBUG_FLAGS; results are WRONG with them): compiled in only with -DPSMF_DEBUG,
@@ -102,7 +102,7 @@ struct KParams {
     void* Yrec; int64_t ldrec; int64_t recsst;
     double* scal_out;
     const double* xbar_ext; const double* F_ext;
-    double* grad_out;         // (n_series, R) accumulated theta gradient or nullptr
+    double* grad_out;         // (n_series, R) accumulated theta gradient, F_GRAD_LINEAR: (n_series, R*R + R) [G_A | G_c]; or nullptr
     double* partials;         // direct kernel: grid_reduce scratch; pipelined kernel: [2][nstat2_pad][pstr] tagged cells
     unsigned long long* bar;  // direct kernel: grid barrier counter; pipelined kernel: [0..1] arrival counters, [2] flag
     long long* status;        // first bad step or -1
@@ -138,6 +138,8 @@ struct KParams {
     const double* rho_mean;   // F_RHO_VECTOR: mean of the caller's diag(R) per series (tr(R)/d of the simplified step)
     const double* lin_A;      // DYN_LINEAR: (r, r) row-major A and (r) offset c (x_bar = A x + c, F = A), device pointers
     const double* lin_c;
+    int64_t glin_off;         // F_GRAD_LINEAR, direct-load and batch kernels: byte offset in dynamic shared memory of the
+                              // accumulator G_A (R * R doubles, row-major); the TMA-staged control CTA uses the start
     unsigned long long spin_ns; // a wait (tagged cell, mbarrier, grid barrier, NVLink mailbox) that makes no progress for
                                 // this long gives up: status word <- STATUS_TIMEOUT | step, abort word (bar[7]) <- 1
 };

@@ -434,6 +434,43 @@ __device__ __forceinline__ double linear_predict(const KParams& p, const double*
     return acc;
 }
 
+// d ell_k / d f_i of the incremental log-likelihood with f = x_bar, N, eta and V held fixed (psmf.py:57-64,167-177;
+// rpsmf.py:62-71,196-200): s = f'Vf + eta = N, e = y - M C f, cte = C'Me, n = n_obs, q = q1
+__device__ __forceinline__ double dll_df(int flags, double vx, double vxt, double cte, double q1, double nobs, double lam, double N) {
+    const double vsf = 0.5 * (vx + vxt);
+    if ((flags & F_LL_STUDENT) != 0) {
+        const double gq = 1.0 + q1 / (lam * N);
+        return nobs * vsf / N - (nobs + lam) / (gq * lam * N) * (cte + (q1 / N) * vsf);
+    }
+    return (nobs / N - q1 / (N * N)) * vsf - cte / N;
+}
+
+// F_GRAD_LINEAR: the accumulator G_A (R * R doubles, row-major) in dynamic shared memory at p.glin_off.  Recomputed where it
+// is used (p lives in the constant bank): no pointer stays live across the row pass.
+__device__ __forceinline__ double* glin_acc(const KParams& p) {
+    extern __shared__ __align__(16) unsigned char psmf_dyn_smem[];
+    return reinterpret_cast<double*>(psmf_dyn_smem + p.glin_off);
+}
+
+// F_GRAD_LINEAR: G_A += gf x_{k-1}' (row-major R x R in shared memory) by one whole warp; lane i < R holds gf_i and
+// x_{k-1, i}.  One FMA per entry and step, in step order, so every kernel, CTA and rank forms the same sum.
+template <int R>
+__device__ __forceinline__ void lin_grad_accum(double* __restrict__ gA, double gf, double xo, int lane) {
+#pragma unroll
+    for (int b = 0; b < R * R; b += 32) {
+        const int idx = b + lane;
+        const double gi = __shfl_sync(FULL, gf, (idx / R) & 31), xj = __shfl_sync(FULL, xo, idx % R);
+        if (idx < R * R) gA[idx] = fma(gi, xj, gA[idx]);
+    }
+}
+
+// end of launch: [G_A row-major | G_c] -> out (R * R + R doubles); G_A was written by another warp
+template <int R>
+__device__ __forceinline__ void lin_grad_writeout(double* __restrict__ out, const double* gA, const double* gc, int tid, int nthr) {
+    __syncthreads();
+    for (int i = tid; i < R * R + R; i += nthr) out[i] = i < R * R ? gA[i] : gc[i - R * R];
+}
+
 // ---- fused evaluation (ExperimentImpute/common.py:79-94) -----------------------------------------------------
 // Accumulated inside the row pass instead of materialising (n, d) Yrec / YrecL / YrecH arrays: over the entries
 // marked in E (the artificially removed ones, Mmiss) the squared one-step prediction error (Epred, rPSMF.py:139) and
@@ -608,12 +645,30 @@ __device__ void gauss_jordan_cta(Smem<R>& sh, int tid) {
     }
 }
 
+// F_GRAD_LINEAR, one whole warp of small_update, after side_half and before x_k replaces x_{k-1}: G_c += gf, G_A += gf x_{k-1}'
+template <int R>
+__device__ __forceinline__ void lin_grad_step(const KParams& p, Smem<R>& sh, const double* tot) {
+    constexpr int NGm = ngram(R);
+    const int lane = threadIdx.x & 31;
+    const bool rhov = (p.flags & F_RHO_VECTOR) != 0;                           // tot is then the nstat_v vector
+    __syncwarp();                                                              // N of side_half (lane 0)
+    double gf = 0.0, xo = 0.0;
+    if (lane < R) {
+        const double cte = rhov ? tot[sv_bu(R) + lane] : tot[NGm + lane] * (sh.rho + sh.a);
+        gf = dll_df(p.flags, sh.vx[lane], sh.vxt[lane], cte, tot[NGm + R + 1], tot[NGm + R + 3], sh.lam, sh.sc[2]);
+        xo = sh.x[lane];
+        sh.grad[lane] += gf;
+    }
+    lin_grad_accum<R>(glin_acc(p), gf, xo, lane);
+}
+
 // ---- r x r part of the step (rPSMF.py:102-115,133-135), identical on every CTA; all `nthr` threads ----
 // Two halves.  eta, N, phi, the update of V and the rank-1 direction g need the reduced statistics but NOT the inverse:
 // when the CTA has a warp outside the NGJ elimination threads (nthr >= NGJ + 32) that warp computes them WHILE the
 // Gauss-Jordan elimination runs; x, omega, P, Q, rho, lambda follow the elimination.  The arithmetic is the same either
 // way (bit-identical results), only the schedule differs.
-template <int R, int NGJ, int BAR = 0, int GJBAR = 1>
+// GL: F_GRAD_LINEAR is set (a template parameter so that the kernels without it compile to the code they had before it)
+template <int R, int NGJ, bool GL = false, int BAR = 0, int GJBAR = 1>
 __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, int warp, int series, int64_t t,
                              bool writer, int nthr, const double* totv = nullptr) {
     constexpr int NGm = ngram(R);
@@ -688,7 +743,12 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
         // the elimination is latency-bound: a subset of the warps runs it (less redundant pivot-search work on
         // the fp64 pipe, cheaper barrier); the first warp past them computes the inverse-free half meanwhile
         if (warp < NGJ / 32) gauss_jordan_cta<R, NGJ, GJBAR>(sh, tid);   // aug[FIN][perm[k]][R..2R) = K[k][:], [..][2R] = (K b)[k]
-        else if (side_warp && warp == NGJ / 32) side_half();
+        else if (side_warp && warp == NGJ / 32) {
+            side_half();
+            // F_GRAD_LINEAR needs N from side_half and the x that entered the step, nothing from the elimination: the side
+            // warp accumulates it while the elimination runs
+            if constexpr (GL) if (p.grad_out != nullptr) lin_grad_step<R>(p, sh, tot);
+        }
         sync_n<BAR>(nthr);
     }
     stamp(p, t, 7);
@@ -696,6 +756,7 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
         if (!side_warp) {
             side_half();
             __syncwarp();
+            if constexpr (GL) if (p.grad_out != nullptr) lin_grad_step<R>(p, sh, tot);
         }
         const double a = sh.a, rho = sh.rho, lam = sh.lam;
         const double s = tot[NGm + R], q1 = tot[NGm + R + 1], nobs = tot[NGm + R + 3];
@@ -717,17 +778,9 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
             sh.x[lane] = xn;
             if (writer && p.X_out != nullptr) p.X_out[((int64_t)series * p.n_steps + t) * R + lane] = xn;
             if (p.grad_out != nullptr && (p.dynamics == DYN_COS || p.dynamics == DYN_EXTERNAL)) {
-                // d ell_k / d theta = J_theta' d ell_k / d f with f = x_bar, s = f'Vf + eta = N, e = y - M C f
-                // (psmf.py:57-64,167-177; rpsmf.py:62-71,196-200); C'Me = b (rho + a), n = n_obs, q = q1
-                const double vsf = 0.5 * (sh.vx[lane] + sh.vxt[lane]);
+                // d ell_k / d theta = J_theta' d ell_k / d f; C'Me = b (rho + a)
                 const double cte = rhov ? tot[sv_bu(R) + lane] : tot[NGm + lane] * (rho + a);
-                double gf;
-                if ((p.flags & F_LL_STUDENT) != 0) {
-                    const double gq = 1.0 + q1 / (lam * N);
-                    gf = nobs * vsf / N - (nobs + lam) / (gq * lam * N) * (cte + (q1 / N) * vsf);
-                } else {
-                    gf = (nobs / N - q1 / (N * N)) * vsf - cte / N;
-                }
+                const double gf = dll_df(p.flags, sh.vx[lane], sh.vxt[lane], cte, q1, nobs, lam, N);
                 const double kabs = (double)(p.k0 + t);
                 // cos dynamics: J_theta = diag(-2 pi k sin(.)); external dynamics: the caller owns f and applies its own
                 // J_theta' to d ell / d f (one step per launch)
@@ -948,7 +1001,7 @@ __device__ __forceinline__ void observe(const KParams& p, const T* __restrict__ 
 // owns them; general fallback (any alignment, any d) and the path for small problems / batched series ----
 // p.phase (caller-driven statistics exchange, one step per launch): 1 = pass + grid reduction, statistics -> p.stats_ext
 // and residuals -> p.e_ext; 2 = r x r update from p.stats_ext (all-reduced by the caller) + the rank-1 update of C.
-template <int R, typename T, bool RHOV = false>
+template <int R, typename T, bool RHOV = false, bool GL = false>
 __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KParams p) {
     constexpr int NW = V1_WARPS, NSP = RHOV ? nstat_v_pad(R) : nstat_pad(R), NST = RHOV ? nstat_v(R) : nstat(R);
     extern __shared__ __align__(16) unsigned char dyn_smem[];
@@ -984,6 +1037,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
         sh.P[i] = stg[st_P(R) + i];
         sh.V[i] = stg[st_V(R) + i];
         sh.Q[i] = stg[st_Q(R) + i];
+        if constexpr (GL) glin_acc(p)[i] = 0.0;
     }
     if (tid < R) {
         sh.x[tid] = stg[st_x(R) + tid];
@@ -1074,7 +1128,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
             for (int e = tid; e < NST; e += blockDim.x) tot_p[e] = p.stats_ext[e];
             __syncthreads();
         }
-        small_update<R, GJ_THREADS>(p, sh, tid, lane, warp, series, t, writer, blockDim.x, RHOV ? totv : nullptr);
+        small_update<R, GJ_THREADS, GL>(p, sh, tid, lane, warp, series, t, writer, blockDim.x, RHOV ? totv : nullptr);
         stamp(p, t, 6);
     }
 
@@ -1099,13 +1153,15 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
         }
         if (tid < R) {
             stg[st_x(R) + tid] = sh.x[tid];
-            if (p.grad_out != nullptr) p.grad_out[(int64_t)series * R + tid] = sh.grad[tid];
+            if (p.grad_out != nullptr && !GL) p.grad_out[(int64_t)series * R + tid] = sh.grad[tid];
         }
         if (tid == 0) {
             stg[st_rho(R)] = sh.rho;
             stg[st_lam(R)] = sh.lam;
         }
     }
+    if constexpr (GL)
+        if (writer && p.grad_out != nullptr) lin_grad_writeout<R>(p.grad_out + (int64_t)series * (R * R + R), glin_acc(p), sh.grad, tid, blockDim.x);
 }
 
 }  // namespace psmf

@@ -12,7 +12,7 @@ namespace psmf {
 
 template <typename T, bool RHOV = false>
 static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t st, bool coop) {
-    auto kern = psmf_filter_kernel<PSMF_R, T, RHOV>;
+    auto kern = (p.flags & F_GRAD_LINEAR) ? psmf_filter_kernel<PSMF_R, T, RHOV, true> : psmf_filter_kernel<PSMF_R, T, RHOV>;
     constexpr int threads = V1_WARPS * 32;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     if (e != cudaSuccess) return e;
@@ -25,6 +25,7 @@ static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t
     return cudaGetLastError();
 }
 
+// the F_GRAD_LINEAR variant has the same launch bounds and static shared memory: its shape is this one's
 template <typename T, bool RHOV = false>
 static cudaError_t shape_t(size_t dyn, LaunchShape* out) {
     auto kern = psmf_filter_kernel<PSMF_R, T, RHOV>;

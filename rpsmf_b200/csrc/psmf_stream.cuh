@@ -656,7 +656,7 @@ __device__ void control_reduce(const KParams& p, ControlSmem<R>& cs) {
 // x and publish {g_t, xbar_{t+1}} as early as possible (that is all the data CTAs wait for); the rest of the
 // r x r update (omega, phi, P, V, Q, rho, lambda, the next predict) follows off the critical path.
 // rPSMF.py:102-115,133-135 with the statistics in the sufficient-statistic form of psmf_filter.cuh.
-template <int R>
+template <int R, bool GL>
 __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
     constexpr int NGm = ngram(R);
     constexpr int NTHR = C_SOLVERS;
@@ -675,6 +675,7 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
         sh.P[i] = stg[st_P(R) + i];
         sh.V[i] = stg[st_V(R) + i];
         sh.Q[i] = stg[st_Q(R) + i];
+        if constexpr (GL) glin_acc(p)[i] = 0.0;
     }
     if (tid < R) {
         sh.x[tid] = stg[st_x(R) + tid];
@@ -894,7 +895,8 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
                 }
             }
             if (!early) stamp(p, t, 6);
-            // (E) off the critical path: omega, phi, gradient of the step log-likelihood
+            // (E) off the critical path: omega, phi, gradient of the step log-likelihood (F_GRAD_LINEAR: with respect to
+            // A and c, from the x_{t-1} still in sh.x)
             const double a = sh.a, rho = sh.rho, lam = sh.lam;
             const double s = sh.tot[NGm + R], q1 = sh.tot[NGm + R + 1], q0 = sh.tot[NGm + R + 2], nobs = sh.tot[NGm + R + 3];
             const double eta = sh.sc[1], N = sh.sc[2];
@@ -902,23 +904,21 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
             const double sSe = s - bkb;                                        // diff' CPinv diff (simplified: s)
             const double omega = robust ? (lam + sSe) / (lam + dg) : 1.0;      // rPSMF.py:105
             const double phi = robust ? (lam + q1 / N + (q0 != 0.0 ? q0 / eta : 0.0)) / (lam + dg) : 1.0;
+            const bool lgrad = GL && p.grad_out != nullptr;
+            double gfl = 0.0, xo = 0.0;
             if (lane < R) {
+                xo = sh.x[lane];
                 sh.x[lane] = xn;
                 if (p.X_out != nullptr) p.X_out[t * R + lane] = xn;
-                if (p.grad_out != nullptr && p.dynamics == DYN_COS) {
-                    // d ell_k / d theta = J_theta' d ell_k / d f (psmf.py:57-64,167-177; rpsmf.py:62-71,196-200)
-                    const double vsf = 0.5 * (sh.vx[lane] + sh.vxt[lane]);
+                if (p.grad_out != nullptr && (p.dynamics == DYN_COS || lgrad)) {
+                    // d ell_k / d theta = J_theta' d ell_k / d f; C'Me = b (rho + a)
                     const double cte = sh.tot[NGm + lane] * (rho + a);
-                    double gf;
-                    if ((p.flags & F_LL_STUDENT) != 0) {
-                        const double gq = 1.0 + q1 / (lam * N);
-                        gf = nobs * vsf / N - (nobs + lam) / (gq * lam * N) * (cte + (q1 / N) * vsf);
-                    } else {
-                        gf = (nobs / N - q1 / (N * N)) * vsf - cte / N;
-                    }
-                    sh.grad[lane] += gf * (6.283185307179586 * (double)(p.k0 + t) * sh.fd[lane]);
+                    const double gf = dll_df(p.flags, sh.vx[lane], sh.vxt[lane], cte, q1, nobs, lam, N);
+                    if (lgrad) gfl = gf;
+                    sh.grad[lane] += lgrad ? gf : gf * (6.283185307179586 * (double)(p.k0 + t) * sh.fd[lane]);
                 }
             }
+            if (lgrad) lin_grad_accum<R>(glin_acc(p), gfl, xo, lane);                // G_c += gf (above), G_A += gf x_{t-1}'
             if (lane == 0) {
                 sh.sc[0] = omega; sh.sc[3] = phi; sh.sc[4] = sSe;
                 sh.sc[5] = p.alpha * phi; sh.sc[6] = p.beta * omega;
@@ -959,11 +959,15 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
     }
     if (tid < R) {
         stg[st_x(R) + tid] = sh.x[tid];
-        if (p.grad_out != nullptr) p.grad_out[tid] = sh.grad[tid];
+        if (p.grad_out != nullptr && !GL) p.grad_out[tid] = sh.grad[tid];
     }
     if (tid == 0) {
         stg[st_rho(R)] = sh.rho;
         stg[st_lam(R)] = sh.lam;
+    }
+    if (GL && p.grad_out != nullptr) {
+        sync_n<CB_S>(NTHR);
+        for (int i = tid; i < R * R + R; i += NTHR) p.grad_out[i] = i < R * R ? glin_acc(p)[i] : sh.grad[i - R * R];
     }
 }
 
@@ -980,7 +984,7 @@ __device__ __forceinline__ void fetch_params(const KParams& p, DataSmem<R>& ps, 
     mbar_wait(p, &ps.par_full[set & 1], (uint32_t)((set >> 1) & 1), set);
 }
 
-template <int R, typename T>
+template <int R, typename T, bool GL = false>
 __global__ void __launch_bounds__(s_threads(), 1) psmf_stream_kernel(const KParams p) {
     if (p.trace != nullptr && threadIdx.x == 0 && (int)blockIdx.x < p.trace_steps) {   // debug: SM id of every CTA (row 159)
         unsigned smid;
@@ -993,7 +997,9 @@ __global__ void __launch_bounds__(s_threads(), 1) psmf_stream_kernel(const KPara
     extern __shared__ __align__(128) unsigned char dyn_smem_s[];
     if (blockIdx.x == gridDim.x - 1) {       // ---- control CTA ----
         ControlSmem<R>& cs = *reinterpret_cast<ControlSmem<R>*>(static_smem);
-        if (uniform_warp_id() < C_SOLVERS / 32) control_solve<R>(p, cs);
+        // F_GRAD_LINEAR: the accumulator G_A is at the start of the control CTA's dynamic shared memory (p.glin_off = 0),
+        // which it has no other use for
+        if (uniform_warp_id() < C_SOLVERS / 32) control_solve<R, GL>(p, cs);
         else control_reduce<R>(p, cs);
         return;
     }

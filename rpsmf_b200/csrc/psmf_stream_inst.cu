@@ -12,7 +12,7 @@ namespace psmf {
 
 template <typename T>
 static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t st, bool coop) {
-    auto kern = psmf_stream_kernel<PSMF_R, T>;
+    auto kern = (p.flags & F_GRAD_LINEAR) ? psmf_stream_kernel<PSMF_R, T, true> : psmf_stream_kernel<PSMF_R, T>;
     constexpr int threads = s_threads();
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     if (e != cudaSuccess) return e;
@@ -25,6 +25,7 @@ static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t
     return cudaGetLastError();
 }
 
+// the F_GRAD_LINEAR variant has the same launch bounds and static shared memory: its shape is this one's
 template <typename T>
 static cudaError_t shape_t(size_t dyn, LaunchShape* out) {
     auto kern = psmf_stream_kernel<PSMF_R, T>;

@@ -24,13 +24,15 @@ def _dev_tensor(a, dtype, device):
 class FilterEngine:
     """One engine = one (batch of) series on one GPU.
 
-    Parameters mirror ``psmf_config`` in include/psmf_b200.h.
+    Parameters mirror ``psmf_config`` in include/psmf_b200.h.  ``grad_linear`` (linear dynamics only) makes
+    ``run(want_grad=True)`` return the gradient of the summed incremental log-likelihood with respect to A and c
+    (``grad_A`` (S, r, r), ``grad_c`` (S, r)) instead of ``grad``.
     """
 
     def __init__(self, d, r, *, n_series=1, dtype=torch.float64, robust=True, simplified=False,
                  c_update_transpose=True, fixed_lambda=False, ll_student=False, dynamics=_capi.DYN_IDENTITY, alpha=1.0,
                  beta=1.0, device=None, d_global=None, world_size=1, rank=0, ctas=0, kernel=0, nan_mask=False,
-                 exchange="nvlink", rho_vector=False):
+                 exchange="nvlink", rho_vector=False, grad_linear=False):
         if not torch.cuda.is_available():
             raise RuntimeError("rpsmf_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         if dtype not in (torch.float64, torch.float32):
@@ -47,6 +49,8 @@ class FilterEngine:
         flags |= _capi.LL_STUDENT if ll_student else 0
         flags |= _capi.NAN_MASK if nan_mask else 0
         flags |= _capi.RHO_VECTOR if rho_vector else 0
+        flags |= _capi.GRAD_LINEAR if grad_linear else 0
+        self.grad_linear = bool(grad_linear)
         self.rho_vector = bool(rho_vector)
         self.nan_mask = bool(nan_mask)
         if exchange not in ("nvlink", "external"):
@@ -173,9 +177,12 @@ class FilterEngine:
             io.scal_out = sc.data_ptr()
             res["scal"] = sc
         if want_grad:
-            gr = torch.zeros((S, r), dtype=torch.float64, device=self.device)
+            gr = torch.zeros((S, r * r + r if self.grad_linear else r), dtype=torch.float64, device=self.device)
             io.grad_out = gr.data_ptr()
-            res["grad"] = gr
+            if self.grad_linear:                      # [G_A row-major | G_c] per series
+                res["grad_A"], res["grad_c"] = gr[:, : r * r].view(S, r, r), gr[:, r * r:]
+            else:
+                res["grad"] = gr
         keep = [Y, M]
         if E is not None:
             if Yorig is None:

@@ -11,6 +11,10 @@ Any other callable ``f(theta, x, t) -> (r, 1)`` is supported through the externa
 evaluates f and its Jacobian once per step and the kernel runs one step per launch (slow, general).
 ``classify`` recognises the two built-ins either by their tag or by probing the callable, so the
 reference's own ``RandomWalk()`` / ``nonlinearity`` objects select the device path unchanged.
+
+A callable that is affine in x, ``f(theta, x, t) = A(theta) x + c(theta)``, can be marked with ``affine(f)``: the
+classes then run it as device linear dynamics (one launch per sweep) and learn theta from the gradient with respect to
+A and c that the kernels accumulate.  Unmarked callables keep the external path.
 """
 
 from __future__ import annotations
@@ -132,3 +136,42 @@ def jacobian_theta(nonlinearity, theta, x, t):
     except Exception:
         pass
     return Jd
+
+
+class affine:
+    """Marks ``f(theta, x, t) = A(theta) x + c(theta)`` (affine in x, independent of t) for the device linear dynamics.
+    Calls go to ``f`` unchanged; ``parts`` checks the claim at a given theta and extracts A and c."""
+
+    _psmf_dynamics = _capi.DYN_LINEAR
+
+    def __init__(self, f):
+        self.f = f
+
+    def __call__(self, theta, x, t):
+        return self.f(theta, x, t)
+
+    def _eval(self, theta, x, t, r):
+        return np.asarray(self.f(theta, np.asarray(x, dtype=np.float64).reshape(r, 1), t), dtype=np.float64).reshape(r)
+
+    def parts(self, theta, r):
+        """(A (r, r), c (r)) at theta: A = [f(theta, e_j) - f(theta, 0)], c = f(theta, 0).  Raises ValueError when f is not
+        affine in x or depends on t at this theta (checked on a few probes)."""
+        eye = np.eye(r)
+        c = self._eval(theta, np.zeros(r), 1, r)
+        A = np.stack([self._eval(theta, eye[j], 1, r) - c for j in range(r)], axis=1)
+        rng = np.random.RandomState(2024)
+        for t in (1, 7, 123):
+            x = rng.randn(r)
+            want = A @ x + c
+            got = self._eval(theta, x, t, r)
+            scale = max(1.0, float(np.max(np.abs(A))) * float(np.max(np.abs(x))) + float(np.max(np.abs(c))))
+            if not np.all(np.isfinite(got)) or np.max(np.abs(got - want)) > 1e-10 * scale:
+                raise ValueError("affine(f): f(theta, x, t) is not A x + c at this theta (not affine in x, or it depends on t)")
+        return A, c
+
+    def theta_jacobians(self, theta, r):
+        """(dA/dtheta (r, r, p), dc/dtheta (r, p)) at theta, from jacobian_theta at x = 0 and x = e_j."""
+        eye = np.eye(r)
+        J0 = jacobian_theta(self.f, theta, np.zeros((r, 1)), 1)
+        dA = np.stack([jacobian_theta(self.f, theta, eye[j].reshape(r, 1), 1) - J0 for j in range(r)], axis=1)
+        return dA, J0

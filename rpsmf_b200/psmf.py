@@ -17,8 +17,11 @@ What differs, by design:
 * R must be rho * I and Q, R constant over k (true for every experiment of the reference); anything else
   raises ``NotImplementedError``.
 * the theta gradient of the incremental likelihood is accumulated on the device in closed form for the
-  built-in ``cos(2 pi theta t + x)`` dynamics (the reference differentiates with autograd); arbitrary
-  callables run through the one-launch-per-step external path without theta learning.
+  built-in ``cos(2 pi theta t + x)`` dynamics (the reference differentiates with autograd).  A callable marked
+  with ``nonlinearities.affine`` (f = A(theta) x + c(theta)) runs as device linear dynamics: A and c are extracted once
+  per sweep (per ``update_every`` block in the Recursive variants), the kernel accumulates the gradient with respect to
+  A and c, and the host closes the chain rule with dA/dtheta, dc/dtheta.  Other callables run through the
+  one-launch-per-step external path, with the theta gradient from the host Jacobian of each step.
 * ``rPSMFIterMissing`` is bound to the masked semantics of ExperimentImpute/rPSMF.py (R_bar = M R M +
   (x'Vx) I), because the class as shipped in the reference is singular for any missing entry
   (SURVEY.md 3.3).
@@ -127,7 +130,8 @@ class PSMFIter:
             self._engine = FilterEngine(
                 self._d, self._r, dtype=self._dtype, robust=self._robust, simplified=self._simplified,
                 c_update_transpose=True, fixed_lambda=getattr(self, "fixed_lambda", False), ll_student=self._ll_student,
-                dynamics=self._dyn, alpha=self._alpha, beta=self._beta, device=self._device, rho_vector=self._rho_vector)
+                dynamics=self._dyn, alpha=self._alpha, beta=self._beta, device=self._device, rho_vector=self._rho_vector,
+                grad_linear=self._dyn == _capi.DYN_LINEAR)
         return self._engine
 
     def _device_y(self, y, T, m=None):
@@ -199,6 +203,16 @@ class PSMFIter:
         if self._dyn == _capi.DYN_EXTERNAL:
             buf[k_first - 1:k_last] = self._sweep_external(eng, ysl, msl, theta, k_first, n)     # accumulates self._gradsum itself
             grad = None
+        elif self._dyn == _capi.DYN_LINEAR:
+            eng.set_linear_dynamics(*self.nonlinearity.parts(theta, self._r))
+            learn = np.asarray(theta).size > 0
+            out = eng.run(ysl, msl, k0=k_first, want_X=False, Yrec_out=buf[k_first - 1:k_last].unsqueeze(0), want_grad=learn)
+            grad = None
+            if learn:
+                # d ell / d theta_p = <dA/dtheta_p, G_A>_F + <dc/dtheta_p, G_c>
+                dA, dc = self.nonlinearity.theta_jacobians(theta, self._r)
+                g = np.einsum("ij,ijp->p", out["grad_A"].cpu().numpy(), dA) + out["grad_c"].cpu().numpy() @ dc
+                self._gradsum = self._gradsum + g.reshape(self._gradsum.shape)
         else:
             out = eng.run(ysl, msl, k0=k_first, want_X=False, Yrec_out=buf[k_first - 1:k_last].unsqueeze(0),
                           want_grad=self._dyn == _capi.DYN_COS)
@@ -275,6 +289,8 @@ class PSMFIter:
             Xo, Yp = eng.predict(n_pred, T + 1, Xpred=np.stack(mus))
         else:
             eng.set_state(theta=self._theta_vec(theta))
+            if self._dyn == _capi.DYN_LINEAR:
+                eng.set_linear_dynamics(*self.nonlinearity.parts(theta, self._r))
             Xo, Yp = eng.predict(n_pred, T + 1)
         Xh = Xo.cpu().numpy()
         Yh = Yp.to(torch.float64).cpu().numpy()
