@@ -61,6 +61,10 @@ typedef struct psmf_engine* psmf_handle;
                                * [G_A = sum_k gf_k x_{k-1}' (r x r row-major) | G_c = sum_k gf_k (r)] per series, gf_k =
                                * d ell_k / d x_bar_k.  d ell / d theta = <dA/dtheta, G_A>_F + <dc/dtheta, G_c> for any A(theta),
                                * c(theta): the caller closes the chain rule.  All kernels; row-sharded ranks agree bit for bit */
+#define PSMF_LOGLIK       512  /* scal_out is PSMF_NSCAL_LL wide and carries the value of the learning objective and the one-step
+                               * predictive log-density of every step (PSMF_SCAL_NLL, PSMF_SCAL_LOGPRED below); nothing is
+                               * computed when scal_out is NULL.  Any flags, dynamics, mask encoding, kernel and sharding;
+                               * row-sharded ranks write bit-identical records.  A non-finite value does not mark the step bad. */
 
 /* dynamics f_theta(x, k) of the predict half (psmf.py:104-115) */
 #define PSMF_DYN_IDENTITY 0    /* RandomWalk, nonlinearities.py:42-56; Impute scripts */
@@ -105,6 +109,26 @@ typedef struct psmf_engine* psmf_handle;
 #define PSMF_SCAL_SSE    5   /* e' S^-1 e                    rPSMF.py:105 */
 #define PSMF_SCAL_LAMBDA 6   /* lambda entering the step */
 #define PSMF_SCAL_RHO    7   /* rho (R = rho I) entering the step */
+/* PSMF_LOGLIK: (n_series, n_steps, PSMF_NSCAL_LL), entries 0..7 as above.  Per step, over the n = n_obs observed rows, with
+ * q1 = sum_obs e_i^2, N = a + eta and lambda entering the step; both are exactly 0 for a step with every row missing.
+ *   PSMF_SCAL_NLL     nll_k, the incremental negative log-likelihood that grad_out differentiates (the d ell_k / d f of
+ *                     PSMF_DYN_COS / PSMF_DYN_EXTERNAL / PSMF_GRAD_LINEAR, with N, eta and V held fixed):
+ *                       Gaussian:               (n/2) log(2 pi N) + q1 / (2 N)
+ *                       PSMF_LL_STUDENT:        lgamma(lambda/2) - lgamma((lambda+n)/2) + (n/2) log(lambda pi N)
+ *                                               + ((lambda+n)/2) log(1 + q1 / (lambda N))
+ *                     i.e. -log of N(y_obs; C_o x_bar, N I) or of the t_lambda density with that scale.  The normalising
+ *                     constants are included; they do not change the gradient.
+ *   PSMF_SCAL_LOGPRED log p(y_obs,k | y_<k) under the filter's own predictive covariance S_obs = C_o Pbar C_o' + diag(rho_i + a):
+ *                       log det S_obs = sum_obs log(rho_i + a) + log det(I + Pbar G)   (matrix-determinant lemma; the second
+ *                                       term from the pivots of the elimination that solves for K, 0 with PSMF_SIMPLIFIED)
+ *                       Delta^2       = diff_obs' S_obs^-1 diff_obs = w1 q1 - b'K b  (PSMF_RHO_VECTOR: sum_obs w_i e_i^2 - b'K b;
+ *                                       PSMF_SIMPLIFIED: S_obs^-1 = diag(w_i), no b'K b)
+ *                       Gaussian:     -(n log(2 pi) + log det S_obs + Delta^2) / 2
+ *                       PSMF_ROBUST:  multivariate t with lambda degrees of freedom: lgamma((lambda+n)/2) - lgamma(lambda/2)
+ *                                     - (n/2) log(lambda pi) - log det S_obs / 2 - ((lambda+n)/2) log(1 + Delta^2 / lambda) */
+#define PSMF_NSCAL_LL     10
+#define PSMF_SCAL_NLL     8
+#define PSMF_SCAL_LOGPRED 9
 
 typedef struct psmf_config {
     int64_t d;          /* rows of C held by this engine (the local shard)                         */
@@ -136,7 +160,7 @@ typedef struct psmf_io {
     void*          Yrec_out;   /* (n_series, n_steps, ldrec) C x_bar (unmasked), or NULL (Yrec, rPSMF.py:89) */
     int64_t        ldrec;
     int64_t        rec_series_stride;
-    double*        scal_out;   /* (n_series, n_steps, PSMF_NSCAL) or NULL                             */
+    double*        scal_out;   /* (n_series, n_steps, PSMF_NSCAL), PSMF_LOGLIK: PSMF_NSCAL_LL; or NULL  */
     const double*  xbar_ext;   /* PSMF_DYN_EXTERNAL: (n_series, r)                                    */
     const double*  F_ext;      /* PSMF_DYN_EXTERNAL: (n_series, r, r) row-major                       */
     double*        grad_out;   /* (n_series, r) sum over the run of d ell_k / d theta (PSMF_DYN_COS), or NULL

@@ -15,10 +15,12 @@ LIB_PATH = os.environ.get("PSMF_B200_LIB") or os.path.join(_HERE, "libpsmf_b200.
 
 F64, F32 = 0, 1
 ROBUST, SIMPLIFIED, CUPDATE_VT, FIXED_LAMBDA, LL_STUDENT, NAN_MASK, RHO_VECTOR, GRAD_LINEAR = 1, 2, 4, 16, 32, 64, 128, 256
+LOGLIK = 512
 DYN_IDENTITY, DYN_COS, DYN_LINEAR, DYN_EXTERNAL = 0, 1, 2, 3
 KERNEL_AUTO, KERNEL_DIRECT, KERNEL_STREAM, KERNEL_BATCH = 0, 1, 2, 3
 XCHG_NVLINK, XCHG_EXTERNAL = 0, 1
 NSCAL = 8
+NSCAL_LL, SCAL_NLL, SCAL_LOGPRED = 10, 8, 9      # LOGLIK: the record gains nll_k and log p(y_obs,k | past)
 NEVAL = 4
 EVAL_SSE, EVAL_INSIDE, EVAL_COUNT = 0, 1, 2
 MAILBOX_BLOB_BYTES = 128

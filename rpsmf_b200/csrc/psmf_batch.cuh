@@ -30,7 +30,7 @@ struct YMreg {
     unsigned char m;
 };
 
-template <int R, typename T, int NW, bool GL = false>
+template <int R, typename T, int NW, bool GL = false, bool LL = false>
 __global__ void __launch_bounds__(NW * 32, batch_min_ctas(R, NW)) psmf_batch_kernel(const KParams p) {
     constexpr int NSP = nstat_pad(R), NST = nstat(R), NTHR = NW * 32;
     // elimination threads: all but one warp, which computes the inverse-free half of the r x r update meanwhile
@@ -69,7 +69,7 @@ __global__ void __launch_bounds__(NW * 32, batch_min_ctas(R, NW)) psmf_batch_ker
         sh.P[i] = stg[st_P(R) + i];
         sh.V[i] = stg[st_V(R) + i];
         sh.Q[i] = stg[st_Q(R) + i];
-        if constexpr (GL) glin_acc(p)[i] = 0.0;
+        if constexpr (GL) if (glin_on<GL, LL>(p)) glin_acc(p)[i] = 0.0;
     }
     if (tid < R) {
         sh.x[tid] = stg[st_x(R) + tid];
@@ -224,7 +224,7 @@ __global__ void __launch_bounds__(NW * 32, batch_min_ctas(R, NW)) psmf_batch_ker
         }
         __syncthreads();
         stamp(p, t, 5);
-        small_update<R, NGJ, GL>(p, sh, tid, lane, warp, series, t, true, NTHR);
+        small_update<R, NGJ, GL, LL>(p, sh, tid, lane, warp, series, t, true, NTHR);
         stamp(p, t, 6);
     }
 
@@ -252,10 +252,10 @@ __global__ void __launch_bounds__(NW * 32, batch_min_ctas(R, NW)) psmf_batch_ker
     }
     if (tid < R) {
         stg[st_x(R) + tid] = sh.x[tid];
-        if (p.grad_out != nullptr && !GL) p.grad_out[(int64_t)series * R + tid] = sh.grad[tid];
+        if (p.grad_out != nullptr && !glin_on<GL, LL>(p)) p.grad_out[(int64_t)series * R + tid] = sh.grad[tid];
     }
     if constexpr (GL)
-        if (p.grad_out != nullptr) lin_grad_writeout<R>(p.grad_out + (int64_t)series * (R * R + R), glin_acc(p), sh.grad, tid, NTHR);
+        if (glin_on<GL, LL>(p) && p.grad_out != nullptr) lin_grad_writeout<R>(p.grad_out + (int64_t)series * (R * R + R), glin_acc(p), sh.grad, tid, NTHR);
     if (tid == 0) {
         stg[st_rho(R)] = sh.rho;
         stg[st_lam(R)] = sh.lam;

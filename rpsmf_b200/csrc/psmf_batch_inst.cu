@@ -12,14 +12,17 @@ namespace psmf {
 
 template <typename T, int NW>
 static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t st) {
-    auto kern = (p.flags & F_GRAD_LINEAR) ? psmf_batch_kernel<PSMF_R, T, NW, true> : psmf_batch_kernel<PSMF_R, T, NW>;
+    // F_LOGLIK: one variant that also serves F_GRAD_LINEAR (glin_on in psmf_filter.cuh)
+    auto kern = (p.flags & F_LOGLIK)        ? psmf_batch_kernel<PSMF_R, T, NW, true, true>
+                : (p.flags & F_GRAD_LINEAR) ? psmf_batch_kernel<PSMF_R, T, NW, true>
+                                            : psmf_batch_kernel<PSMF_R, T, NW>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     if (e != cudaSuccess) return e;
     kern<<<grid, NW * 32, dyn, st>>>(p);
     return cudaGetLastError();
 }
 
-// the F_GRAD_LINEAR variant has the same launch bounds and static shared memory: its shape is this one's
+// the F_GRAD_LINEAR and F_LOGLIK variants have the same launch bounds and static shared memory: its shape is this one's
 template <typename T, int NW>
 static cudaError_t shape_t(size_t dyn, LaunchShape* out) {
     auto kern = psmf_batch_kernel<PSMF_R, T, NW>;

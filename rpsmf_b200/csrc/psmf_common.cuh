@@ -16,12 +16,13 @@ namespace psmf {
 
 constexpr int TILE = 32;
 constexpr int NSCAL = 8;
+constexpr int NSCAL_LL = 10;   // F_LOGLIK: the record gains [nll_k, log p_k] (include/psmf_b200.h PSMF_SCAL_NLL / PSMF_SCAL_LOGPRED)
 constexpr int MAXR = 16;
 constexpr int MAX_PEERS = 8;
 
 // flags (mirror include/psmf_b200.h)
 constexpr int F_ROBUST = 1, F_SIMPLIFIED = 2, F_CUPDATE_VT = 4, F_FIXED_LAMBDA = 16, F_LL_STUDENT = 32, F_NAN_MASK = 64,
-              F_RHO_VECTOR = 128, F_GRAD_LINEAR = 256;
+              F_RHO_VECTOR = 128, F_GRAD_LINEAR = 256, F_LOGLIK = 512;
 constexpr int DYN_IDENTITY = 0, DYN_COS = 1, DYN_LINEAR = 2, DYN_EXTERNAL = 3;
 constexpr int NEVAL = 4;     // fused evaluation record (include/psmf_b200.h PSMF_EVAL_*)
 // debug-only flag bits (env PSMF_DEBUG_FLAGS; results are WRONG with them): compiled in only with -DPSMF_DEBUG,
@@ -69,6 +70,9 @@ __host__ __device__ constexpr int nstat_v_pad(int R) { return (nstat_v(R) + 7) /
 __host__ __device__ constexpr int sv_G0(int R) { return ngram(R) + R + 4; }
 __host__ __device__ constexpr int sv_bu(int R) { return 2 * ngram(R) + R + 4; }
 __host__ __device__ constexpr int sv_nrho(int R) { return 2 * ngram(R) + 2 * R + 4; }
+// F_RHO_VECTOR with F_LOGLIK: one more entry behind them, sum m log(rho_i + a) (the diagonal part of log det S_obs).  nstat_v(R)
+// is odd, so the padding always has room for it: buffers sized by nstat_v_pad hold it.
+__host__ __device__ constexpr int sv_nlog(int R) { return nstat_v(R); }
 // packed index of Gram entry (j, j) in row-major upper-triangular order
 __host__ __device__ constexpr int gram_off(int R, int j) { return j * R - j * (j - 1) / 2; }
 // tagged 16-byte cells behind KParams.gparams: [2][2 MAXR] parameter sets, then [2][nstat2_pad(MAXR)] reduced totals

@@ -38,7 +38,8 @@ struct Smem {
     double g[R];        // rank-1 direction of the previous step
     double th[R];
     double P[R * R], V[R * R], Q[R * R], Pb[R * R];
-    double aug[2][R][2 * R + 2];   // double-buffered augmented matrix of the r x r solve
+    double aug[2][R][2 * R + 2];   // double-buffered augmented matrix of the r x r solve; column 2R + 1 is padding, where
+                                   // F_LOGLIK keeps the pivot of elimination step k: aug[0][k][2R + 1]
     double tot[NSP];
     double part[NSP];
     double a, rho, lam;
@@ -445,6 +446,40 @@ __device__ __forceinline__ double dll_df(int flags, double vx, double vxt, doubl
     return (nobs / N - q1 / (N * N)) * vsf - cte / N;
 }
 
+// F_LOGLIK: nll_k and log p_k of one step (include/psmf_b200.h PSMF_LOGLIK), by one whole warp; every lane returns both.
+//   n = n_obs, N = a + eta, q1 = sum_obs e^2, lam = lambda entering the step, ldr = sum_obs log(rho_i + a),
+//   d2 = Delta^2 = diff_obs' S_obs^-1 diff_obs (w1 q1 - b'Kb);
+//   lane i < R holds pivot i of the elimination of I + Pbar G (1.0 on the other lanes and without an elimination):
+//   log det S_obs = ldr + sum_i log|pivot_i| (matrix-determinant lemma; det(I + Pbar G) >= 1, so no sign to track).
+// The transcendentals of the different terms are the same instruction on different lanes, and the pivot sum has a fixed
+// order: every CTA and every rank gets the same bits.
+__device__ __forceinline__ void step_loglik(int flags, double piv, double n, double N, double q1, double lam, double ldr, double d2,
+                                            int lane, double& nll, double& lp) {
+    constexpr double PI = 3.141592653589793;
+    const double lgdet = warp_allsum(log(fabs(piv)));
+    const double lg = lgamma(0.5 * (lane == 1 ? lam + n : lam));                    // lane 0: lgamma(lam/2), 1: lgamma((lam+n)/2)
+    const double lv = log(((lane & 1) ? lam : 2.0) * PI * (lane < 2 ? N : 1.0));    // lane 0: log 2piN, 1: log lam pi N, 2: log 2pi,
+                                                                                    // 3: log lam pi
+    const double l1 = log1p(lane == 0 ? q1 / (lam * N) : d2 / lam);                 // lane 0: log(1 + q1/(lam N)), 1: log(1 + d2/lam)
+    const double lg0 = __shfl_sync(FULL, lg, 0), lg1 = __shfl_sync(FULL, lg, 1);
+    const double l2piN = __shfl_sync(FULL, lv, 0), llpiN = __shfl_sync(FULL, lv, 1);
+    const double l2pi = __shfl_sync(FULL, lv, 2), llpi = __shfl_sync(FULL, lv, 3);
+    const double lq = __shfl_sync(FULL, l1, 0), ld = __shfl_sync(FULL, l1, 1);
+    const double logdet = ldr + lgdet;
+    if (n == 0.0) {                                                                 // every row missing: no observation, no term
+        nll = 0.0;
+        lp = 0.0;
+        return;
+    }
+    nll = (flags & F_LL_STUDENT) != 0 ? (lg0 - lg1) + 0.5 * n * llpiN + 0.5 * (lam + n) * lq : 0.5 * n * l2piN + q1 / (2.0 * N);
+    lp = (flags & F_ROBUST) != 0 ? (lg1 - lg0) - 0.5 * n * llpi - 0.5 * logdet - 0.5 * (lam + n) * ld : -0.5 * (n * l2pi + logdet + d2);
+}
+
+// The F_LOGLIK variant (LL) of each kernel serves F_GRAD_LINEAR too (GL = true, the flag decides at run time): one more
+// instantiation per kernel instead of the GL x LL product.  In the GL-only variant this is a constant, so it compiles as before.
+template <bool GL, bool LL>
+__device__ __forceinline__ bool glin_on(const KParams& p) { return GL && (!LL || (p.flags & F_GRAD_LINEAR) != 0); }
+
 // F_GRAD_LINEAR: the accumulator G_A (R * R doubles, row-major) in dynamic shared memory at p.glin_off.  Recomputed where it
 // is used (p lives in the constant bank): no pointer stays live across the row pass.
 __device__ __forceinline__ double* glin_acc(const KParams& p) {
@@ -596,9 +631,10 @@ __device__ void predict_cta(const KParams& p, Smem<R>& sh, int tid, int64_t k, i
 // column k and the pivot row of the previous step.  Rows are not swapped: step k eliminates with the unused
 // row of largest |a_ik| -- found redundantly by every warp (no broadcast barrier) with one warp-wide
 // integer max over the high words of |a_ik| (16 mantissa bits decide, ties -> lowest row) -- and perm[k]
-// remembers it, so the solution row of unknown k is aug[R & 1][perm[k]].
+// remembers it, so the solution row of unknown k is aug[R & 1][perm[k]].  PIV (F_LOGLIK): the writer of perm[k] also keeps
+// the pivot a_{perm[k], k} in aug[0][k][2R + 1] (a padding column) for log det(I + Pbar G).
 constexpr int GJ_THREADS = 192;                         // direct-load kernel; the pipelined kernel uses its control warps
-template <int R, int NGJ, int GJBAR = 1, int NC = 2 * R + 1>
+template <int R, int NGJ, int GJBAR = 1, int NC = 2 * R + 1, bool PIV = false>
 __device__ void gauss_jordan_cta(Smem<R>& sh, int tid) {
     constexpr int TPR = NGJ / R;                        // threads per row
     constexpr int CPT = (NC + TPR - 1) / TPR;           // columns per thread
@@ -625,7 +661,10 @@ __device__ void gauss_jordan_cta(Smem<R>& sh, int tid) {
         const int pi = 15 - (__reduce_max_sync(FULL, key) & 15);
         const double inv = __shfl_sync(FULL, cinv, pi);
         used |= 1u << pi;
-        if (tid == 0) sh.perm[k] = pi;
+        if (tid == 0) {
+            sh.perm[k] = pi;
+            if constexpr (PIV) sh.aug[0][k][2 * R + 1] = sh.aug[cur][pi][k];
+        }
         // all pivot-row loads first: the stores below may alias them as far as the compiler can tell, and
         // interleaving would serialise load -> multiply -> store per column
         double rp[CPT];
@@ -667,8 +706,9 @@ __device__ __forceinline__ void lin_grad_step(const KParams& p, Smem<R>& sh, con
 // when the CTA has a warp outside the NGJ elimination threads (nthr >= NGJ + 32) that warp computes them WHILE the
 // Gauss-Jordan elimination runs; x, omega, P, Q, rho, lambda follow the elimination.  The arithmetic is the same either
 // way (bit-identical results), only the schedule differs.
-// GL: F_GRAD_LINEAR is set (a template parameter so that the kernels without it compile to the code they had before it)
-template <int R, int NGJ, bool GL = false, int BAR = 0, int GJBAR = 1>
+// GL: F_GRAD_LINEAR is set, LL: F_LOGLIK is set (template parameters so that the kernels without them compile to the code they
+// had before them; see glin_on)
+template <int R, int NGJ, bool GL = false, bool LL = false, int BAR = 0, int GJBAR = 1>
 __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, int warp, int series, int64_t t,
                              bool writer, int nthr, const double* totv = nullptr) {
     constexpr int NGm = ngram(R);
@@ -742,12 +782,12 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
         sync_n<BAR>(nthr);
         // the elimination is latency-bound: a subset of the warps runs it (less redundant pivot-search work on
         // the fp64 pipe, cheaper barrier); the first warp past them computes the inverse-free half meanwhile
-        if (warp < NGJ / 32) gauss_jordan_cta<R, NGJ, GJBAR>(sh, tid);   // aug[FIN][perm[k]][R..2R) = K[k][:], [..][2R] = (K b)[k]
+        if (warp < NGJ / 32) gauss_jordan_cta<R, NGJ, GJBAR, 2 * R + 1, LL>(sh, tid);   // aug[FIN][perm[k]][R..2R) = K[k][:], [..][2R] = (K b)[k]
         else if (side_warp && warp == NGJ / 32) {
             side_half();
             // F_GRAD_LINEAR needs N from side_half and the x that entered the step, nothing from the elimination: the side
             // warp accumulates it while the elimination runs
-            if constexpr (GL) if (p.grad_out != nullptr) lin_grad_step<R>(p, sh, tot);
+            if constexpr (GL) if (glin_on<GL, LL>(p) && p.grad_out != nullptr) lin_grad_step<R>(p, sh, tot);
         }
         sync_n<BAR>(nthr);
     }
@@ -756,7 +796,7 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
         if (!side_warp) {
             side_half();
             __syncwarp();
-            if constexpr (GL) if (p.grad_out != nullptr) lin_grad_step<R>(p, sh, tot);
+            if constexpr (GL) if (glin_on<GL, LL>(p) && p.grad_out != nullptr) lin_grad_step<R>(p, sh, tot);
         }
         const double a = sh.a, rho = sh.rho, lam = sh.lam;
         const double s = tot[NGm + R], q1 = tot[NGm + R + 1], nobs = tot[NGm + R + 3];
@@ -791,11 +831,27 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
             sh.sc[0] = omega; sh.sc[4] = sSe; sh.sc[6] = p.beta * omega;
             if (writer) {
                 if (p.scal_out != nullptr) {
-                    double* so = p.scal_out + ((int64_t)series * p.n_steps + t) * NSCAL;
+                    double* so = p.scal_out + ((int64_t)series * p.n_steps + t) * (LL ? NSCAL_LL : NSCAL);
                     so[0] = a; so[1] = eta; so[2] = N; so[3] = omega; so[4] = phi; so[5] = sSe; so[6] = lam; so[7] = rho;
                 }
                 if (!(isfinite(N) && isfinite(omega) && isfinite(phi) && isfinite(xn)) || N == 0.0)
                     atomicCAS((unsigned long long*)p.status, ~0ULL, (unsigned long long)t);
+            }
+        }
+        if constexpr (LL) {
+            if (p.scal_out != nullptr) {
+                // S_obs = C_o Pbar C_o' + diag(rho_i + a): log det from the pivots and sum_obs log(rho_i + a), Delta^2 = s over
+                // the observed rows - b'Kb (s also carries w0 q0 of the missing rows; simplified: S_obs^-1 = diag(w_i), b'Kb = 0)
+                const double q0 = tot[NGm + R + 2];
+                const double piv = (!simp && lane < R) ? sh.aug[0][lane][2 * R + 1] : 1.0;
+                const double ldr = rhov ? tot[sv_nlog(R)] : nobs * log(rho + a);
+                const double d2 = (rhov ? s - (q0 != 0.0 ? sh.w0 * q0 : 0.0) : sh.w1 * q1) - bkb;
+                double nll, lp;
+                step_loglik(p.flags, piv, nobs, N, q1, lam, ldr, d2, lane, nll, lp);
+                if (lane == 0 && writer) {
+                    double* so = p.scal_out + ((int64_t)series * p.n_steps + t) * NSCAL_LL;
+                    so[8] = nll; so[9] = lp;
+                }
             }
         }
     }
@@ -1001,9 +1057,11 @@ __device__ __forceinline__ void observe(const KParams& p, const T* __restrict__ 
 // owns them; general fallback (any alignment, any d) and the path for small problems / batched series ----
 // p.phase (caller-driven statistics exchange, one step per launch): 1 = pass + grid reduction, statistics -> p.stats_ext
 // and residuals -> p.e_ext; 2 = r x r update from p.stats_ext (all-reduced by the caller) + the rank-1 update of C.
-template <int R, typename T, bool RHOV = false, bool GL = false>
+template <int R, typename T, bool RHOV = false, bool GL = false, bool LL = false>
 __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KParams p) {
-    constexpr int NW = V1_WARPS, NSP = RHOV ? nstat_v_pad(R) : nstat_pad(R), NST = RHOV ? nstat_v(R) : nstat(R);
+    // RHOV with LL: one more statistic, sum m log(rho_i + a), inside the padding
+    constexpr int NW = V1_WARPS, NSP = RHOV ? nstat_v_pad(R) : nstat_pad(R), NST = RHOV ? nstat_v(R) + (LL ? 1 : 0) : nstat(R);
+    static_assert(NST <= NSP, "statistics vector longer than its padded size");
     extern __shared__ __align__(16) unsigned char dyn_smem[];
     __shared__ Smem<R> sh;
     __shared__ double red[V1_WARPS * NSP];                                     // per-warp partial statistics
@@ -1037,7 +1095,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
         sh.P[i] = stg[st_P(R) + i];
         sh.V[i] = stg[st_V(R) + i];
         sh.Q[i] = stg[st_Q(R) + i];
-        if constexpr (GL) glin_acc(p)[i] = 0.0;
+        if constexpr (GL) if (glin_on<GL, LL>(p)) glin_acc(p)[i] = 0.0;
     }
     if (tid < R) {
         sh.x[tid] = stg[st_x(R) + tid];
@@ -1068,6 +1126,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
             if constexpr (RHOV) acc.zero_v(); else acc.zero();
             const double* __restrict__ rho0 = RHOV ? p.rho_vec + (int64_t)series * p.rho_sst : nullptr;
             const double rscale = sh.rho, aa = sh.a;
+            double nlog = 0.0;                                                     // RHOV && LL: sum m log(rho_i + a)
             for (int tile = tb + warp; tile < te; tile += NW) {
                 const int64_t row = (int64_t)tile * TILE + lane;
                 const int rl = (tile - tb) * TILE + lane;
@@ -1087,6 +1146,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
                     const double rho_i = inb ? __dmul_rn(rscale, rho0[row]) : 1.0;       // R = omega-scale * diag(R0)  (rPSMF.py:134)
                     wi = 1.0 / (rho_i + aa);                                               // rPSMF.py:92,98,32
                     acc.nrho += mi ? rho_i : 0.0;
+                    if constexpr (LL) if (p.scal_out != nullptr) nlog += mi ? log(rho_i + aa) : 0.0;
                 }
                 row_stats<R>(acc, sh, c, ep, inb, mi, yi, wi, w0, e, yh);
 #pragma unroll
@@ -1105,6 +1165,10 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
             }
             if constexpr (RHOV) acc_writeout_v<R>(acc, red + warp * NSP, lane);
             else acc_writeout<R>(acc, red + warp * NSP, w1, lane);
+            if constexpr (RHOV && LL) {
+                const double nl = warp_allsum(nlog);
+                if (lane == 0) red[warp * NSP + sv_nlog(R)] = nl;
+            }
             stamp(p, t, 1);
             __syncthreads();
             stamp(p, t, 2);
@@ -1128,7 +1192,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
             for (int e = tid; e < NST; e += blockDim.x) tot_p[e] = p.stats_ext[e];
             __syncthreads();
         }
-        small_update<R, GJ_THREADS, GL>(p, sh, tid, lane, warp, series, t, writer, blockDim.x, RHOV ? totv : nullptr);
+        small_update<R, GJ_THREADS, GL, LL>(p, sh, tid, lane, warp, series, t, writer, blockDim.x, RHOV ? totv : nullptr);
         stamp(p, t, 6);
     }
 
@@ -1153,7 +1217,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
         }
         if (tid < R) {
             stg[st_x(R) + tid] = sh.x[tid];
-            if (p.grad_out != nullptr && !GL) p.grad_out[(int64_t)series * R + tid] = sh.grad[tid];
+            if (p.grad_out != nullptr && !glin_on<GL, LL>(p)) p.grad_out[(int64_t)series * R + tid] = sh.grad[tid];
         }
         if (tid == 0) {
             stg[st_rho(R)] = sh.rho;
@@ -1161,7 +1225,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
         }
     }
     if constexpr (GL)
-        if (writer && p.grad_out != nullptr) lin_grad_writeout<R>(p.grad_out + (int64_t)series * (R * R + R), glin_acc(p), sh.grad, tid, blockDim.x);
+        if (writer && glin_on<GL, LL>(p) && p.grad_out != nullptr) lin_grad_writeout<R>(p.grad_out + (int64_t)series * (R * R + R), glin_acc(p), sh.grad, tid, blockDim.x);
 }
 
 }  // namespace psmf

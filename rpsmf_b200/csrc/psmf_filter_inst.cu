@@ -12,7 +12,10 @@ namespace psmf {
 
 template <typename T, bool RHOV = false>
 static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t st, bool coop) {
-    auto kern = (p.flags & F_GRAD_LINEAR) ? psmf_filter_kernel<PSMF_R, T, RHOV, true> : psmf_filter_kernel<PSMF_R, T, RHOV>;
+    // F_LOGLIK: one variant that also serves F_GRAD_LINEAR (glin_on in psmf_filter.cuh)
+    auto kern = (p.flags & F_LOGLIK)        ? psmf_filter_kernel<PSMF_R, T, RHOV, true, true>
+                : (p.flags & F_GRAD_LINEAR) ? psmf_filter_kernel<PSMF_R, T, RHOV, true>
+                                            : psmf_filter_kernel<PSMF_R, T, RHOV>;
     constexpr int threads = V1_WARPS * 32;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     if (e != cudaSuccess) return e;
@@ -25,7 +28,7 @@ static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t
     return cudaGetLastError();
 }
 
-// the F_GRAD_LINEAR variant has the same launch bounds and static shared memory: its shape is this one's
+// the F_GRAD_LINEAR and F_LOGLIK variants have the same launch bounds and static shared memory: its shape is this one's
 template <typename T, bool RHOV = false>
 static cudaError_t shape_t(size_t dyn, LaunchShape* out) {
     auto kern = psmf_filter_kernel<PSMF_R, T, RHOV>;

@@ -656,7 +656,7 @@ __device__ void control_reduce(const KParams& p, ControlSmem<R>& cs) {
 // x and publish {g_t, xbar_{t+1}} as early as possible (that is all the data CTAs wait for); the rest of the
 // r x r update (omega, phi, P, V, Q, rho, lambda, the next predict) follows off the critical path.
 // rPSMF.py:102-115,133-135 with the statistics in the sufficient-statistic form of psmf_filter.cuh.
-template <int R, bool GL>
+template <int R, bool GL, bool LL>
 __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
     constexpr int NGm = ngram(R);
     constexpr int NTHR = C_SOLVERS;
@@ -675,7 +675,7 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
         sh.P[i] = stg[st_P(R) + i];
         sh.V[i] = stg[st_V(R) + i];
         sh.Q[i] = stg[st_Q(R) + i];
-        if constexpr (GL) glin_acc(p)[i] = 0.0;
+        if constexpr (GL) if (glin_on<GL, LL>(p)) glin_acc(p)[i] = 0.0;
     }
     if (tid < R) {
         sh.x[tid] = stg[st_x(R) + tid];
@@ -743,7 +743,7 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
         // (C) elimination (C_GJ threads) next to the side computations (two warps)
         if (warp < C_GJ / 32) {
             // aug[FIN][perm[k]][R..2R) = K[k][:]   (measured: 128 and 192 threads tie at 2.3 us, 64: 5.8, 32: 9.1)
-            if (!simp) gauss_jordan_cta<R, C_GJ, CB_GJ, 2 * R>(sh, tid);
+            if (!simp) gauss_jordan_cta<R, C_GJ, CB_GJ, 2 * R, LL>(sh, tid);
         } else if (warp == C_GJ / 32) {
             // b = w1 (h - A xbar), q1 = gamma - 2 xbar'h + xbar'A xbar, s = w1 q1 + w0 q0
             double ax = 0.0, hj = 0.0, xj = 0.0;
@@ -896,7 +896,7 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
             }
             if (!early) stamp(p, t, 6);
             // (E) off the critical path: omega, phi, gradient of the step log-likelihood (F_GRAD_LINEAR: with respect to
-            // A and c, from the x_{t-1} still in sh.x)
+            // A and c, from the x_{t-1} still in sh.x), F_LOGLIK: its value and the one-step predictive log-density
             const double a = sh.a, rho = sh.rho, lam = sh.lam;
             const double s = sh.tot[NGm + R], q1 = sh.tot[NGm + R + 1], q0 = sh.tot[NGm + R + 2], nobs = sh.tot[NGm + R + 3];
             const double eta = sh.sc[1], N = sh.sc[2];
@@ -904,7 +904,7 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
             const double sSe = s - bkb;                                        // diff' CPinv diff (simplified: s)
             const double omega = robust ? (lam + sSe) / (lam + dg) : 1.0;      // rPSMF.py:105
             const double phi = robust ? (lam + q1 / N + (q0 != 0.0 ? q0 / eta : 0.0)) / (lam + dg) : 1.0;
-            const bool lgrad = GL && p.grad_out != nullptr;
+            const bool lgrad = glin_on<GL, LL>(p) && p.grad_out != nullptr;
             double gfl = 0.0, xo = 0.0;
             if (lane < R) {
                 xo = sh.x[lane];
@@ -923,11 +923,22 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
                 sh.sc[0] = omega; sh.sc[3] = phi; sh.sc[4] = sSe;
                 sh.sc[5] = p.alpha * phi; sh.sc[6] = p.beta * omega;
                 if (p.scal_out != nullptr) {
-                    double* so = p.scal_out + t * NSCAL;
+                    double* so = p.scal_out + t * (LL ? NSCAL_LL : NSCAL);
                     so[0] = a; so[1] = eta; so[2] = N; so[3] = omega; so[4] = phi; so[5] = sSe; so[6] = lam; so[7] = rho;
                 }
                 if (!(isfinite(N) && isfinite(omega) && isfinite(phi) && isfinite(xn)) || N == 0.0)
                     atomicCAS((unsigned long long*)p.status, ~0ULL, (unsigned long long)t);
+            }
+            if constexpr (LL) {
+                if (p.scal_out != nullptr) {           // as in small_update (psmf_filter.cuh), uniform R
+                    const double piv = (!simp && lane < R) ? sh.aug[0][lane][2 * R + 1] : 1.0;
+                    double nll, lp;
+                    step_loglik(p.flags, piv, nobs, N, q1, lam, nobs * log(rho + a), sh.w1 * q1 - bkb, lane, nll, lp);
+                    if (lane == 0) {
+                        p.scal_out[t * NSCAL_LL + 8] = nll;
+                        p.scal_out[t * NSCAL_LL + 9] = lp;
+                    }
+                }
             }
             __syncwarp();
         }
@@ -959,13 +970,13 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
     }
     if (tid < R) {
         stg[st_x(R) + tid] = sh.x[tid];
-        if (p.grad_out != nullptr && !GL) p.grad_out[tid] = sh.grad[tid];
+        if (p.grad_out != nullptr && !glin_on<GL, LL>(p)) p.grad_out[tid] = sh.grad[tid];
     }
     if (tid == 0) {
         stg[st_rho(R)] = sh.rho;
         stg[st_lam(R)] = sh.lam;
     }
-    if (GL && p.grad_out != nullptr) {
+    if (glin_on<GL, LL>(p) && p.grad_out != nullptr) {
         sync_n<CB_S>(NTHR);
         for (int i = tid; i < R * R + R; i += NTHR) p.grad_out[i] = i < R * R ? glin_acc(p)[i] : sh.grad[i - R * R];
     }
@@ -984,7 +995,7 @@ __device__ __forceinline__ void fetch_params(const KParams& p, DataSmem<R>& ps, 
     mbar_wait(p, &ps.par_full[set & 1], (uint32_t)((set >> 1) & 1), set);
 }
 
-template <int R, typename T, bool GL = false>
+template <int R, typename T, bool GL = false, bool LL = false>
 __global__ void __launch_bounds__(s_threads(), 1) psmf_stream_kernel(const KParams p) {
     if (p.trace != nullptr && threadIdx.x == 0 && (int)blockIdx.x < p.trace_steps) {   // debug: SM id of every CTA (row 159)
         unsigned smid;
@@ -999,7 +1010,7 @@ __global__ void __launch_bounds__(s_threads(), 1) psmf_stream_kernel(const KPara
         ControlSmem<R>& cs = *reinterpret_cast<ControlSmem<R>*>(static_smem);
         // F_GRAD_LINEAR: the accumulator G_A is at the start of the control CTA's dynamic shared memory (p.glin_off = 0),
         // which it has no other use for
-        if (uniform_warp_id() < C_SOLVERS / 32) control_solve<R, GL>(p, cs);
+        if (uniform_warp_id() < C_SOLVERS / 32) control_solve<R, GL, LL>(p, cs);
         else control_reduce<R>(p, cs);
         return;
     }

@@ -12,7 +12,10 @@ namespace psmf {
 
 template <typename T>
 static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t st, bool coop) {
-    auto kern = (p.flags & F_GRAD_LINEAR) ? psmf_stream_kernel<PSMF_R, T, true> : psmf_stream_kernel<PSMF_R, T>;
+    // F_LOGLIK: one variant that also serves F_GRAD_LINEAR (glin_on in psmf_filter.cuh)
+    auto kern = (p.flags & F_LOGLIK)        ? psmf_stream_kernel<PSMF_R, T, true, true>
+                : (p.flags & F_GRAD_LINEAR) ? psmf_stream_kernel<PSMF_R, T, true>
+                                            : psmf_stream_kernel<PSMF_R, T>;
     constexpr int threads = s_threads();
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     if (e != cudaSuccess) return e;
@@ -25,7 +28,7 @@ static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t
     return cudaGetLastError();
 }
 
-// the F_GRAD_LINEAR variant has the same launch bounds and static shared memory: its shape is this one's
+// the F_GRAD_LINEAR and F_LOGLIK variants have the same launch bounds and static shared memory: its shape is this one's
 template <typename T>
 static cudaError_t shape_t(size_t dyn, LaunchShape* out) {
     auto kern = psmf_stream_kernel<PSMF_R, T>;

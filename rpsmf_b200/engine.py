@@ -26,13 +26,16 @@ class FilterEngine:
 
     Parameters mirror ``psmf_config`` in include/psmf_b200.h.  ``grad_linear`` (linear dynamics only) makes
     ``run(want_grad=True)`` return the gradient of the summed incremental log-likelihood with respect to A and c
-    (``grad_A`` (S, r, r), ``grad_c`` (S, r)) instead of ``grad``.
+    (``grad_A`` (S, r, r), ``grad_c`` (S, r)) instead of ``grad``.  ``loglik`` makes the per-step scalar record 10 wide:
+    ``run(want_loglik=True)`` returns ``nll`` (the incremental negative log-likelihood that the gradients differentiate) and
+    ``logpred`` (the one-step predictive log-density log p(y_obs,k | y_<k)), each (S, T) float64 (include/psmf_b200.h
+    PSMF_LOGLIK).
     """
 
     def __init__(self, d, r, *, n_series=1, dtype=torch.float64, robust=True, simplified=False,
                  c_update_transpose=True, fixed_lambda=False, ll_student=False, dynamics=_capi.DYN_IDENTITY, alpha=1.0,
                  beta=1.0, device=None, d_global=None, world_size=1, rank=0, ctas=0, kernel=0, nan_mask=False,
-                 exchange="nvlink", rho_vector=False, grad_linear=False):
+                 exchange="nvlink", rho_vector=False, grad_linear=False, loglik=False):
         if not torch.cuda.is_available():
             raise RuntimeError("rpsmf_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
         if dtype not in (torch.float64, torch.float32):
@@ -50,6 +53,8 @@ class FilterEngine:
         flags |= _capi.NAN_MASK if nan_mask else 0
         flags |= _capi.RHO_VECTOR if rho_vector else 0
         flags |= _capi.GRAD_LINEAR if grad_linear else 0
+        flags |= _capi.LOGLIK if loglik else 0
+        self.loglik = bool(loglik)
         self.grad_linear = bool(grad_linear)
         self.rho_vector = bool(rho_vector)
         self.nan_mask = bool(nan_mask)
@@ -134,13 +139,17 @@ class FilterEngine:
 
     # -- the hot path ------------------------------------------------------------------------------
     def run(self, Y, M=None, k0=1, want_X=True, want_Yrec=False, want_scal=False, xbar=None, F=None,
-            X_out=None, Yrec_out=None, scal_out=None, want_grad=False, Yorig=None, E=None, sig=2.0, _finish=False):
+            X_out=None, Yrec_out=None, scal_out=None, want_grad=False, Yorig=None, E=None, sig=2.0, want_loglik=False,
+            _finish=False):
         """Filter ``T`` steps.  Y: device tensor (T, d) or (S, T, d) in the engine dtype (last dim may be
         padded: ld = stride of the time axis); M: uint8 tensor of the same shape or None.
 
         Fused evaluation (common.py:79-94): with ``E`` (uint8, 1 = evaluate here: the artificially removed entries)
         and ``Yorig`` (original values, same shape and strides as Y) the result holds ``eval`` = (S, 4) sums over this
-        run: [sum (y_hat - y_orig)^2, entries inside y_hat -+ sig sqrt(U), entries of E, 0]."""
+        run: [sum (y_hat - y_orig)^2, entries inside y_hat -+ sig sqrt(U), entries of E, 0].
+
+        ``want_loglik`` (an engine created with ``loglik=True``): ``nll`` and ``logpred``, (S, T) views of the 10-wide scalar
+        record, which ``scal`` then is."""
         S, d, r = self.S, self.d, self.r
         if not isinstance(Y, torch.Tensor) or Y.device != self.device:
             raise ValueError("Y must be a tensor on %s" % self.device)
@@ -172,10 +181,17 @@ class FilterEngine:
                 Yr = Yr.unsqueeze(0)
             io.Yrec_out, io.ldrec, io.rec_series_stride = Yr.data_ptr(), Yr.stride(1), Yr.stride(0)
             res["Yrec"] = Yr
-        if want_scal or scal_out is not None:
-            sc = scal_out if scal_out is not None else torch.empty((S, T, _capi.NSCAL), dtype=torch.float64, device=self.device)
+        if want_loglik and not self.loglik:
+            raise ValueError("want_loglik needs an engine created with loglik=True")
+        if want_scal or want_loglik or scal_out is not None:
+            nsc = _capi.NSCAL_LL if self.loglik else _capi.NSCAL
+            sc = scal_out if scal_out is not None else torch.empty((S, T, nsc), dtype=torch.float64, device=self.device)
+            if self.loglik and (sc.shape[-1] != nsc or not sc.is_contiguous()):
+                raise ValueError("scal_out of a loglik engine must be a contiguous (S, T, %d) tensor" % nsc)
             io.scal_out = sc.data_ptr()
             res["scal"] = sc
+            if want_loglik:
+                res["nll"], res["logpred"] = sc[..., _capi.SCAL_NLL], sc[..., _capi.SCAL_LOGPRED]
         if want_grad:
             gr = torch.zeros((S, r * r + r if self.grad_linear else r), dtype=torch.float64, device=self.device)
             io.grad_out = gr.data_ptr()

@@ -25,6 +25,10 @@ What differs, by design:
 * ``rPSMFIterMissing`` is bound to the masked semantics of ExperimentImpute/rPSMF.py (R_bar = M R M +
   (x'Vx) I), because the class as shipped in the reference is singular for any missing entry
   (SURVEY.md 3.3).
+* ``loglik=True`` (keyword-only, all classes): sweep i also records ``_objective[i]`` = sum_k nll_k, the summed incremental
+  negative log-likelihood whose gradient the optimisers descend, and ``_logpred[i]`` = sum_k log p(y_k | y_<k), the
+  one-step predictive log-likelihood, both computed in the filter kernel (include/psmf_b200.h PSMF_LOGLIK).  The Recursive
+  variants make one sweep: key 1, summed over their ``update_every`` blocks.
 """
 
 from __future__ import annotations
@@ -79,7 +83,7 @@ class PSMFIter:
     _ll_student = False
 
     def __init__(self, theta0, C0, V0, mu0, P0, Qs, Rs, nonlinearity, optim="adam", simplified=False, device=None,
-                 dtype=torch.float64):
+                 dtype=torch.float64, *, loglik=False):
         self.nonlinearity = nonlinearity
         assert optim in ["adam", "sgd"]
         self.optim = optim
@@ -114,6 +118,10 @@ class PSMFIter:
         self._alpha = 1.0
         self._beta = 1.0
         self._gradsum = np.zeros(np.asarray(theta0).shape)
+        self._loglik = bool(loglik)
+        self._objective = {}
+        self._logpred = {}
+        self._llsum = None
 
     # ---- configuration handed to the kernel ----------------------------------------------------------
     def _q_rho(self):
@@ -131,7 +139,7 @@ class PSMFIter:
                 self._d, self._r, dtype=self._dtype, robust=self._robust, simplified=self._simplified,
                 c_update_transpose=True, fixed_lambda=getattr(self, "fixed_lambda", False), ll_student=self._ll_student,
                 dynamics=self._dyn, alpha=self._alpha, beta=self._beta, device=self._device, rho_vector=self._rho_vector,
-                grad_linear=self._dyn == _capi.DYN_LINEAR)
+                grad_linear=self._dyn == _capi.DYN_LINEAR, loglik=self._loglik)
         return self._engine
 
     def _device_y(self, y, T, m=None):
@@ -172,7 +180,21 @@ class PSMFIter:
 
     def step(self, y, i, T):
         self.step_reset()
+        self._loglik_begin()
         self._sweep(y, None, self._theta[i - 1], 1, T)
+        self._loglik_store(i)
+
+    def _loglik_begin(self):
+        self._llsum = None
+
+    def _add_loglik(self, out):
+        if self._loglik:
+            s = torch.stack([out["nll"].sum(), out["logpred"].sum()])       # on the device: no transfer per block
+            self._llsum = s if self._llsum is None else self._llsum + s
+
+    def _loglik_store(self, i):
+        if self._loglik:
+            self._objective[i], self._logpred[i] = (self._llsum.tolist() if self._llsum is not None else [0.0, 0.0])
 
     def _sweep(self, y, m, theta, k_first, k_last, materialize=True):
         """Filter steps k_first..k_last (1-based, inclusive) with a fixed theta; state dicts move from
@@ -206,7 +228,9 @@ class PSMFIter:
         elif self._dyn == _capi.DYN_LINEAR:
             eng.set_linear_dynamics(*self.nonlinearity.parts(theta, self._r))
             learn = np.asarray(theta).size > 0
-            out = eng.run(ysl, msl, k0=k_first, want_X=False, Yrec_out=buf[k_first - 1:k_last].unsqueeze(0), want_grad=learn)
+            out = eng.run(ysl, msl, k0=k_first, want_X=False, Yrec_out=buf[k_first - 1:k_last].unsqueeze(0), want_grad=learn,
+                          want_loglik=self._loglik)
+            self._add_loglik(out)
             grad = None
             if learn:
                 # d ell / d theta_p = <dA/dtheta_p, G_A>_F + <dc/dtheta_p, G_c>
@@ -215,7 +239,8 @@ class PSMFIter:
                 self._gradsum = self._gradsum + g.reshape(self._gradsum.shape)
         else:
             out = eng.run(ysl, msl, k0=k_first, want_X=False, Yrec_out=buf[k_first - 1:k_last].unsqueeze(0),
-                          want_grad=self._dyn == _capi.DYN_COS)
+                          want_grad=self._dyn == _capi.DYN_COS, want_loglik=self._loglik)
+            self._add_loglik(out)
             grad = out.get("grad")
         bad = eng.status()
         if bad >= 0:
@@ -251,7 +276,8 @@ class PSMFIter:
             xbar = np.asarray(self.nonlinearity(theta, x, k), dtype=np.float64).reshape(self._r)
             F = None if self._simplified else jacobian_x(self.nonlinearity, theta, x, k)
             out = eng.run(ysl[j:j + 1], None if msl is None else msl[j:j + 1], k0=k, want_X=False, Yrec_out=Yrec[j:j + 1],
-                          xbar=xbar, F=F, want_grad=learn)
+                          xbar=xbar, F=F, want_grad=learn, want_loglik=self._loglik)
+            self._add_loglik(out)
             if learn:
                 # d ell_k / d theta = J_theta' d ell_k / d f  (psmf.py:167-177): the kernel returns d ell_k / d f
                 gf = out["grad"].cpu().numpy().reshape(self._r)
@@ -365,6 +391,7 @@ class _RecursiveMixin:
 
     def step(self, y, T):
         self.step_reset()
+        self._loglik_begin()
         k = 1
         ue = max(1, int(self._update_every))
         while k <= T:
@@ -379,6 +406,7 @@ class _RecursiveMixin:
             else:
                 self._carry_theta(k_last)
             k = k_last + 1
+        self._loglik_store(1)
 
     def _reset_gradient(self):
         self._gradsum = np.zeros(np.asarray(self.theta0).shape)

@@ -18,10 +18,10 @@ class rPSMFIter(PSMFIter):
     _ll_student = True
 
     def __init__(self, theta0, C0, V0, mu0, P0, Q0, R0, lambda0, nonlinearity, fixed_lambda=False, use_scaling=False,
-                 optim="adam", simplified=False, device=None, dtype=torch.float64):
+                 optim="adam", simplified=False, device=None, dtype=torch.float64, *, loglik=False):
         assert optim in ["adam", "sgd"]
         super().__init__(theta0, C0, V0, mu0, P0, Q0, R0, nonlinearity, optim=optim, simplified=simplified,
-                         device=device, dtype=dtype)
+                         device=device, dtype=dtype, loglik=loglik)
         self.Q0 = Q0
         self.R0 = R0
         self.lambda0 = lambda0
@@ -105,7 +105,9 @@ class rPSMFIterMissing(rPSMFIter):
 
     def step(self, y, m, i, T):
         self.step_reset()
+        self._loglik_begin()
         self._sweep(y, m, self._theta[i - 1], 1, T)
+        self._loglik_store(i)
 
 
 class rPSMFRecursive(_RecursiveMixin, rPSMFIter):
