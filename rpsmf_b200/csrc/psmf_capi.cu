@@ -278,7 +278,20 @@ extern "C" int psmf_create(psmf_handle* out, const psmf_config* cfg) {
         free_engine(e);
         return fail(nullptr, PSMF_E_NOMEM, "d too large: per-CTA residual buffer exceeds shared memory");
     }
-    if (e->S == 1 && cps > 1 && cps > sms * shp.max_ctas_per_sm) cps = sms * shp.max_ctas_per_sm;
+    // a forced grid larger than what fits on the device at once is cut to the co-resident count (cooperative launch);
+    // fewer CTAs hold more tiles each, so the residual buffer is sized again for the grid that runs, until it is stable
+    // (a larger buffer can lower the occupancy once more)
+    while (e->S == 1 && cps > 1 && cps > sms * shp.max_ctas_per_sm) {
+        cps = sms * shp.max_ctas_per_sm;
+        const int64_t tiles_per = (e->ntiles + cps - 1) / cps + 1;
+        e->dyn_smem = stage_bytes + (size_t)tiles_per * TILE * sizeof(double);
+        ce = ((cfg->flags & PSMF_RHO_VECTOR) ? SHAPE_V : SHAPE)[e->R](cfg->dtype, e->dyn_smem, &shp);
+        if (ce != cudaSuccess || shp.max_ctas_per_sm < 1) {
+            cudaGetLastError();
+            free_engine(e);
+            return fail(nullptr, PSMF_E_NOMEM, "d too large: per-CTA residual buffer exceeds shared memory");
+        }
+    }
     e->cps = cps;
     e->threads = shp.threads;
     e->cooperative = cps > 1;

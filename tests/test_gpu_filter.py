@@ -36,12 +36,12 @@ def _padded(a, dtype, dev, pad=0, gap=0, fill=0):
 
 
 def _engine_run(d, r, Y, M, C0, x0, init, robust, ctas=0, dtype=None, chunks=None, S=None, pad=0, gap=0, rec_pad=0,
-                want_grad=False, Yorig=None, E=None, **kw):
+                want_grad=False, Yorig=None, E=None, sig=2.0, **kw):
     """Run the engine over Y (T, d), or (S, T, d) with S series, in the launches given by `chunks`.  `pad` / `gap` put Y, M
     (and Yorig, E) inside larger buffers (rows of d + pad elements, gaps between series); `rec_pad` writes Yrec into rows
     of d + rec_pad elements whose padding is NaN and must stay so.  Returns (X, Yrec, scal, state, launch_info); with S
     the arrays keep the series axis, the state holds the theta gradient ("grad", summed over the launches) when
-    `want_grad` and the fused evaluation sums ("eval") when E is given."""
+    `want_grad` and the fused evaluation sums ("eval", coverage of yhat -+ sig sqrt(U)) when E is given."""
     torch = _torch()
     from rpsmf_b200 import FilterEngine
     dtype = dtype or torch.float64
@@ -62,7 +62,7 @@ def _engine_run(d, r, Y, M, C0, x0, init, robust, ctas=0, dtype=None, chunks=Non
     for a, b in zip(bounds[:-1], bounds[1:]):
         out = eng.run(Yd[:, a:b], None if Md is None else Md[:, a:b], k0=1 + a, want_X=True, Yrec_out=Yrec[:, a:b],
                       want_scal=True, want_grad=want_grad, Yorig=None if Yod is None else Yod[:, a:b],
-                      E=None if Ed is None else Ed[:, a:b])
+                      E=None if Ed is None else Ed[:, a:b], sig=sig)
         assert eng.status() == -1
         Xs.append(out["X"].reshape(Sn, b - a, r).cpu().numpy()); Sc.append(out["scal"].reshape(Sn, b - a, -1).cpu().numpy())
         if want_grad:
@@ -86,10 +86,10 @@ def _engine_run(d, r, Y, M, C0, x0, init, robust, ctas=0, dtype=None, chunks=Non
     return X, Yr, Sc, st, info
 
 
-def _oracle_run(Y, M, C0, x0, init, cfg, k0=1):
+def _oracle_run(Y, M, C0, x0, init, cfg, k0=1, record=None):
     st = po.OracleState(C0.copy(), x0.copy(), init["P"].copy(), init["V"].copy(), init["Q"].copy(), init["rho"],
                         init["lam"], init.get("theta"))
-    return po.run(st, cfg, Y, None if M is None else M.astype(float), k0=k0)
+    return po.run(st, cfg, Y, None if M is None else M.astype(float), k0=k0, record=record)
 
 
 def _compare(res, ref, tol):
