@@ -55,7 +55,8 @@ typedef struct psmf_engine* psmf_handle;
 
 #define PSMF_RHO_VECTOR   128  /* R is diagonal but NOT uniform (psmf.py:144-152 takes the Woodbury branch for any diagonal R; the
                                * flat functions accept any (d, d) R): `rho` of psmf_set_state / psmf_get_state is then
-                               * (n_series, d) = diag(R).  One GPU, direct-load kernel.                                */
+                               * (n_series, d) = diag(R).  One GPU, direct-load kernel.
+                               * Not with PSMF_XCHG_EXTERNAL (psmf_create refuses it): that exchange shards by rows. */
 #define PSMF_GRAD_LINEAR  256  /* PSMF_DYN_LINEAR only: grad_out is the gradient of the summed incremental log-likelihood with
                                * respect to A and c (x_bar = A x + c, N, eta and V held fixed, as for the cos gradient):
                                * [G_A = sum_k gf_k x_{k-1}' (r x r row-major) | G_c = sum_k gf_k (r)] per series, gf_k =

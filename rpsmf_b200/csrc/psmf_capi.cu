@@ -219,6 +219,11 @@ extern "C" int psmf_create(psmf_handle* out, const psmf_config* cfg) {
     if ((cfg->flags & PSMF_RHO_VECTOR) && (cfg->world_size > 1 || cfg->kernel == 2 || cfg->kernel == 3))
         return fail(nullptr, PSMF_E_INVALID, "PSMF_RHO_VECTOR (non-uniform diagonal R) runs on the direct-load kernel of one GPU: "
                                              "world_size 1, kernel AUTO or DIRECT");
+    // the caller-driven exchange exists to shard one series by rows, which a non-uniform R does not support; its longer
+    // statistics vector (nstat_v) would not fit the exchange buffer nor match the count psmf_stats_buffer reports
+    if ((cfg->flags & PSMF_RHO_VECTOR) && cfg->exchange == PSMF_XCHG_EXTERNAL)
+        return fail(nullptr, PSMF_E_INVALID, "PSMF_RHO_VECTOR (non-uniform diagonal R) runs on one GPU without row sharding: "
+                                             "not with PSMF_XCHG_EXTERNAL");
     if ((cfg->flags & PSMF_GRAD_LINEAR) && cfg->dynamics != PSMF_DYN_LINEAR)
         return fail(nullptr, PSMF_E_INVALID, "PSMF_GRAD_LINEAR is the gradient with respect to A and c: it needs PSMF_DYN_LINEAR");
     if (cfg->exchange == PSMF_XCHG_EXTERNAL && cfg->n_series > 1)

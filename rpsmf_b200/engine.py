@@ -217,6 +217,8 @@ class FilterEngine:
             res["eval"] = ev
             keep += [Yorig, E]
         if self.dynamics == _capi.DYN_EXTERNAL:
+            if xbar is None:
+                raise ValueError("external dynamics: every run needs xbar (and F unless simplified)")
             xb = _dev_tensor(xbar, torch.float64, self.device).reshape(S, r)
             io.xbar_ext = xb.data_ptr()
             keep.append(xb)
@@ -310,11 +312,21 @@ class FilterEngine:
     def run_split(self, Y, M, k0, allreduce, **kw):
         """One filter step with the exchange done by the caller: pass + reduction of this GPU's rows, ``allreduce(buf)``
         (in place, sum over the GPUs that share the series; e.g. ``torch.distributed.all_reduce`` = ncclAllReduce on the
-        current stream), then the r x r update and the rank-1 update of C."""
+        current stream), then the r x r update and the rank-1 update of C.  Takes the keywords of ``run``.
+
+        The pass writes the reconstruction, so ``Yrec_out`` / ``want_Yrec`` go to the first launch; X, the scalar record and
+        the gradients come from the second.  External dynamics (``xbar``, ``F``) are read by both."""
         buf = self.stats_buffer()
-        self.run(Y, M, k0=k0, want_X=False)
+        dyn = {k: kw[k] for k in ("xbar", "F") if k in kw}
+        rec = kw.pop("Yrec_out", None)
+        if kw.pop("want_Yrec", False) and rec is None:
+            rec = torch.empty((self.S, Y.shape[-2], self.d), dtype=self.dtype, device=self.device)
+        first = self.run(Y, M, k0=k0, want_X=False, Yrec_out=rec, **dyn)
         allreduce(buf)
-        return self.run(Y, M, k0=k0, _finish=True, **kw)
+        out = self.run(Y, M, k0=k0, _finish=True, **kw)
+        if rec is not None:
+            out["Yrec"] = first["Yrec"]
+        return out
 
     # -- dynamics, forecast, evaluation ------------------------------------------------------------------
     def set_linear_dynamics(self, A, c=None):
