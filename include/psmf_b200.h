@@ -142,7 +142,11 @@ typedef struct psmf_config {
     int32_t device;     /* CUDA device ordinal                                                      */
     int32_t world_size; /* GPUs sharing ONE series by rows (1 = no exchange)                       */
     int32_t rank;
-    int32_t ctas;       /* CTAs per series, 0 = auto                                                */
+    int32_t ctas;       /* CTAs per series, 0 = auto.  n_series > 1: the cluster size of a series (1..16): one CTA
+                         * per series while a series fits it (auto), else a thread-block cluster of ctas CTAs per
+                         * series that reduces through distributed shared memory -- an ordinary launch, not
+                         * cooperative, so the clusters run in waves when the device cannot hold them all; auto
+                         * picks the size from the row count, the number of series and what the device schedules */
     int32_t kernel;     /* PSMF_KERNEL_* (error if the forced kernel is not eligible for the shape)         */
     double  alpha;      /* V scale (rpsmf.py:45-51), 1.0 unless use_scaling                        */
     double  beta;       /* P scale                                                                  */
@@ -237,7 +241,8 @@ int  psmf_count_nan(int32_t device, int32_t dtype, const void* Y, int64_t ldy, i
  * different kernel; the launch has then drained with invalid results instead of hanging.              */
 int  psmf_status(psmf_handle h, int64_t* first_bad_step);
 
-/* introspection used by bench.py / tests, describing the last psmf_run: CTAs per series, threads per CTA,
+/* introspection used by bench.py / tests, describing the last psmf_run: CTAs per series (n_series > 1 and the
+ * direct-load kernel: ctas > 1 is the cluster path), threads per CTA,
  * dynamic smem bytes, kernels launched, which kernel ran (PSMF_KERNEL_*) and, for the TMA-staged kernel, its
  * shared-memory chunk slots and whether C stayed resident in shared memory.                          */
 int  psmf_launch_info(psmf_handle h, int32_t* ctas, int32_t* threads, int32_t* smem_bytes, int32_t* launches);

@@ -49,6 +49,15 @@ static const shape_fn SHAPE_B8[MAXR + 1] = {
     nullptr,          shape_batch8_r1,  shape_batch8_r2,  shape_batch8_r3,  shape_batch8_r4,  shape_batch8_r5,
     shape_batch8_r6,  shape_batch8_r7,  shape_batch8_r8,  shape_batch8_r9,  shape_batch8_r10, shape_batch8_r11,
     shape_batch8_r12, shape_batch8_r13, shape_batch8_r14, shape_batch8_r15, shape_batch8_r16};
+static const launch_c_fn LAUNCH_C[MAXR + 1] = {
+    nullptr,            launch_filterc_r1,  launch_filterc_r2,  launch_filterc_r3,  launch_filterc_r4,  launch_filterc_r5,
+    launch_filterc_r6,  launch_filterc_r7,  launch_filterc_r8,  launch_filterc_r9,  launch_filterc_r10, launch_filterc_r11,
+    launch_filterc_r12, launch_filterc_r13, launch_filterc_r14, launch_filterc_r15, launch_filterc_r16};
+static const shape_c_fn SHAPE_C[MAXR + 1] = {
+    nullptr,           shape_filterc_r1,  shape_filterc_r2,  shape_filterc_r3,  shape_filterc_r4,  shape_filterc_r5,
+    shape_filterc_r6,  shape_filterc_r7,  shape_filterc_r8,  shape_filterc_r9,  shape_filterc_r10, shape_filterc_r11,
+    shape_filterc_r12, shape_filterc_r13, shape_filterc_r14, shape_filterc_r15, shape_filterc_r16};
+constexpr int MAX_CLUSTER = 16;     // CTAs of one series in a cluster (sizes above 8 are non-portable: the device decides)
 static size_t batch_dyn(int64_t ntiles, int R, size_t esize, bool eval) { return batch_dyn_bytes(ntiles, R, esize, eval); }
 static const shape_fn SHAPE[MAXR + 1] = {
     nullptr,          shape_filter_r1,  shape_filter_r2,  shape_filter_r3,  shape_filter_r4,  shape_filter_r5,
@@ -128,6 +137,7 @@ struct psmf_engine {
     int cps = 1, threads = 0, launches_last = 0, num_sms = 0;
     size_t dyn_smem = 0;
     bool cooperative = false;
+    bool cluster = false;              // n_series > 1 with cps > 1: one thread-block cluster of cps CTAs per series (not cooperative)
     // TMA-staged kernel configuration (cps2 == 0: not available for this shape)
     int cps2 = 0, threads2 = 0, nslot = 0;
     size_t dyn_smem2 = 0;
@@ -203,6 +213,68 @@ static void free_engine(psmf_engine* e) {
     delete e;
 }
 
+// n_series > 1, a series over a cluster of CTAs of the direct-load kernel: `want` CTAs (2..16), or 0 for the automatic size.
+// Sets e->cps and e->dyn_smem (stage tiles + residual buffer; run_impl appends the evaluation buffers, G_A and the cluster's
+// partial statistics behind it).
+static int plan_cluster(psmf_engine* e, int want, size_t stage_bytes, LaunchShape* shp) {
+    const bool rhov = (e->cfg.flags & PSMF_RHO_VECTOR) != 0;
+    const size_t pub = cluster_pub_bytes(e->R, rhov);
+    auto dyn_for = [&](int c) { return stage_bytes + (size_t)((e->ntiles + c - 1) / c + 1) * TILE * sizeof(double); };
+    // fits: one CTA with this buffer fits an SM; returns whether the device can hold one cluster of c such CTAs
+    auto sched = [&](int c, bool* fits) {
+        int ncl = 0;
+        const bool ok = SHAPE_C[e->R](e->cfg.dtype, rhov, dyn_for(c) + pub, c, shp, &ncl) == cudaSuccess && shp->max_ctas_per_sm >= 1;
+        cudaGetLastError();
+        if (fits) *fits = ok;
+        return ok && ncl >= 1;
+    };
+    int c;
+    if (want > 0) {
+        c = want > e->ntiles ? (int)e->ntiles : want;
+        if (!sched(c, nullptr))
+            return fail(nullptr, PSMF_E_NOMEM, "n_series > 1: the device cannot schedule a cluster of " + std::to_string(c) +
+                                                   " CTAs per series at d = " + std::to_string(e->d) + " (per-CTA residual buffer of " +
+                                                   std::to_string((e->ntiles + c - 1) / c + 1) + " tiles)");
+    } else {
+        int c_min = 0, c_max = 0;
+        for (int k = 2; k <= MAX_CLUSTER; ++k) {
+            bool fits = false;
+            if (sched(k, &fits)) c_max = k;
+            if (fits && c_min == 0) c_min = k;
+        }
+        if (c_min == 0 || c_max == 0 || c_min > c_max) {
+            // rows one series can have: the largest cluster the device schedules with CTAs whose residual buffers fill their
+            // shared memory
+            int ncl = 0, lim = 0;
+            LaunchShape s0;
+            SHAPE_C[e->R](e->cfg.dtype, rhov, 0, 2, &s0, &ncl);
+            cudaGetLastError();
+            const int64_t tiles = ((int64_t)e->maxsmem - s0.static_smem - (int64_t)(stage_bytes + pub)) / (TILE * (int64_t)sizeof(double)) - 1;
+            for (int k = 2; tiles > 0 && k <= MAX_CLUSTER; ++k) {
+                LaunchShape sk;
+                if (SHAPE_C[e->R](e->cfg.dtype, rhov, stage_bytes + (size_t)(tiles + 1) * TILE * sizeof(double) + pub, k, &sk, &ncl) ==
+                        cudaSuccess && sk.max_ctas_per_sm >= 1 && ncl >= 1)
+                    lim = k;
+                cudaGetLastError();
+            }
+            return fail(nullptr, PSMF_E_NOMEM, "d too large for a batched engine: a series runs on a cluster of at most " + std::to_string(lim) +
+                                                   " CTAs here, which holds about " + std::to_string(lim * (tiles > 0 ? tiles : 0) * TILE) +
+                                                   " rows at r = " + std::to_string(e->R) + " (d = " + std::to_string(e->d) +
+                                                   "); create one engine per series");
+        }
+        c = e->num_sms / e->S;
+        if (c > c_max) c = c_max;
+        if (c > e->ntiles) c = (int)e->ntiles;
+        if (c < c_min) c = c_min;
+        while (c < c_max && !sched(c, nullptr)) ++c;    // a size between the two that the device cannot schedule: the next one
+        if (!sched(c, nullptr)) return fail(nullptr, PSMF_E_NOMEM, "n_series > 1: no schedulable cluster size for this d");
+    }
+    e->cps = c;
+    e->dyn_smem = dyn_for(c);
+    e->cluster = true;
+    return PSMF_OK;
+}
+
 extern "C" int psmf_create(psmf_handle* out, const psmf_config* cfg) {
     if (!out || !cfg) return fail(nullptr, PSMF_E_INVALID, "null argument");
     *out = nullptr;
@@ -257,7 +329,13 @@ extern "C" int psmf_create(psmf_handle* out, const psmf_config* cfg) {
     }
 
     // ---- direct-load kernel: V1_WARPS warps per CTA, one staging tile per warp + the residual buffer ----
+    // n_series > 1: one CTA per series while that fits, else (or with ctas >= 2) a thread-block cluster of CTAs per series
+    if (e->S > 1 && cfg->ctas > MAX_CLUSTER) {
+        free_engine(e);
+        return fail(nullptr, PSMF_E_INVALID, "n_series > 1: ctas is the cluster size of a series, 1..16");
+    }
     int cps;
+    bool cluster = e->S > 1 && cfg->ctas >= 2 && e->ntiles >= 2;
     if (e->S > 1) {
         cps = 1;
     } else if (cfg->ctas > 0) {
@@ -269,7 +347,7 @@ extern "C" int psmf_create(psmf_handle* out, const psmf_config* cfg) {
     if ((int64_t)cps > e->ntiles) cps = (int)e->ntiles;
     const size_t stage_bytes = (size_t)V1_WARPS * e->R * TILE * sizeof(double);
     LaunchShape shp;
-    for (;;) {
+    for (; !cluster;) {
         const int64_t tiles_per = (e->ntiles + cps - 1) / cps + 1;
         e->dyn_smem = stage_bytes + (size_t)tiles_per * TILE * sizeof(double);
         ce = ((cfg->flags & PSMF_RHO_VECTOR) ? SHAPE_V : SHAPE)[e->R](cfg->dtype, e->dyn_smem, &shp);
@@ -279,6 +357,10 @@ extern "C" int psmf_create(psmf_handle* out, const psmf_config* cfg) {
         if (e->S == 1 && cfg->ctas <= 0 && cps < sms) {
             cps = cps * 2 > sms ? sms : cps * 2;
             continue;
+        }
+        if (e->S > 1 && cfg->ctas <= 0) {
+            cluster = true;
+            break;
         }
         free_engine(e);
         return fail(nullptr, PSMF_E_NOMEM, "d too large: per-CTA residual buffer exceeds shared memory");
@@ -298,8 +380,15 @@ extern "C" int psmf_create(psmf_handle* out, const psmf_config* cfg) {
         }
     }
     e->cps = cps;
+    if (cluster) {
+        const int rc = plan_cluster(e, cfg->ctas >= 2 ? cfg->ctas : 0, stage_bytes, &shp);
+        if (rc != PSMF_OK) {
+            free_engine(e);
+            return rc;
+        }
+    }
     e->threads = shp.threads;
-    e->cooperative = cps > 1;
+    e->cooperative = e->cps > 1 && !e->cluster;
 
     // ---- TMA-staged kernel: slots of v2_ts(R, esize) tiles, residual buffer behind them ----
     if ((cfg->kernel == 0 || cfg->kernel == 2) && !(cfg->flags & PSMF_RHO_VECTOR) && cfg->exchange == PSMF_XCHG_NVLINK &&
@@ -622,19 +711,33 @@ static int run_impl(psmf_handle h, const psmf_io* io, int64_t n_steps, int64_t k
         h->last_dyn = h->dyn_smem2;
     } else {
         size_t dyn1 = h->dyn_smem;
+        const bool rhov = (h->cfg.flags & PSMF_RHO_VECTOR) != 0;
         if (eval || glin) {
             const int64_t tiles_per = (h->ntiles + h->cps - 1) / h->cps + 1;
             if (eval) dyn1 += (size_t)tiles_per * TILE * 17 + 16;
             p.glin_off = (int64_t)dyn1;
             dyn1 += glin;
             LaunchShape sh1;
-            if (((h->cfg.flags & PSMF_RHO_VECTOR) ? SHAPE_V : SHAPE)[h->R](h->cfg.dtype, dyn1, &sh1) != cudaSuccess || sh1.max_ctas_per_sm < 1 ||
-                (h->cooperative && h->cps > h->num_sms * sh1.max_ctas_per_sm)) {
+            if (!h->cluster && (((h->cfg.flags & PSMF_RHO_VECTOR) ? SHAPE_V : SHAPE)[h->R](h->cfg.dtype, dyn1, &sh1) != cudaSuccess || sh1.max_ctas_per_sm < 1 ||
+                (h->cooperative && h->cps > h->num_sms * sh1.max_ctas_per_sm))) {
                 cudaGetLastError();
                 return fail(h, PSMF_E_NOMEM, "no shared memory left for the evaluation buffers / the gradient accumulator at this d / grid");
             }
         }
-        CK(h, ((h->cfg.flags & PSMF_RHO_VECTOR) ? LAUNCH_V : LAUNCH)[h->R](p, h->cfg.dtype, h->S * h->cps, dyn1, st, h->cooperative));
+        if (h->cluster) {
+            // the partial statistics the peers read go last (psmf_filter.cuh grid_reduce); the device must still hold one cluster
+            dyn1 += cluster_pub_bytes(h->R, rhov);
+            LaunchShape sh1;
+            int ncl = 0;
+            if (SHAPE_C[h->R](h->cfg.dtype, rhov, dyn1, h->cps, &sh1, &ncl) != cudaSuccess || sh1.max_ctas_per_sm < 1 || ncl < 1) {
+                cudaGetLastError();
+                return fail(h, PSMF_E_NOMEM, "no shared memory left for the evaluation buffers / the gradient accumulator in a cluster of " +
+                                                 std::to_string(h->cps) + " CTAs at this d");
+            }
+            CK(h, LAUNCH_C[h->R](p, h->cfg.dtype, rhov, h->S * h->cps, dyn1, st, h->cps));
+        } else {
+            CK(h, (rhov ? LAUNCH_V : LAUNCH)[h->R](p, h->cfg.dtype, h->S * h->cps, dyn1, st, h->cooperative));
+        }
         h->last_kernel = 1;
         h->last_dyn = dyn1;
     }

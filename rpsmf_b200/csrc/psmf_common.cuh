@@ -171,6 +171,11 @@ struct LaunchShape {
 // per-R entry points, one translation unit each (psmf_filter_inst.cu compiled with -DPSMF_R=n)
 typedef cudaError_t (*launch_fn)(const KParams&, int dtype, int grid, size_t dyn_smem, cudaStream_t, bool cooperative);
 typedef cudaError_t (*shape_fn)(int dtype, size_t dyn_smem, LaunchShape*);
+// cluster variant of the direct-load kernel (batched engines): grid = n_series * csize, clusters of csize CTAs; its dynamic
+// shared memory ends with the parity-double-buffered partial statistics that the peers of the cluster read
+typedef cudaError_t (*launch_c_fn)(const KParams&, int dtype, bool rhov, int grid, size_t dyn_smem, cudaStream_t, int csize);
+typedef cudaError_t (*shape_c_fn)(int dtype, bool rhov, size_t dyn_smem, int csize, LaunchShape*, int* max_clusters);
+__host__ __device__ constexpr size_t cluster_pub_bytes(int R, bool rhov) { return (size_t)2 * (rhov ? nstat_v_pad(R) : nstat_pad(R)) * 8; }
 
 }  // namespace psmf
 
@@ -180,6 +185,8 @@ typedef cudaError_t (*shape_fn)(int dtype, size_t dyn_smem, LaunchShape*);
     cudaError_t shape_filter_r##n(int, size_t, LaunchShape*);                                               \
     cudaError_t launch_filterv_r##n(const KParams&, int, int, size_t, cudaStream_t, bool);                  \
     cudaError_t shape_filterv_r##n(int, size_t, LaunchShape*);                                              \
+    cudaError_t launch_filterc_r##n(const KParams&, int, bool, int, size_t, cudaStream_t, int);             \
+    cudaError_t shape_filterc_r##n(int, bool, size_t, int, LaunchShape*, int*);                             \
     cudaError_t launch_stream_r##n(const KParams&, int, int, size_t, cudaStream_t, bool);                   \
     cudaError_t shape_stream_r##n(int, size_t, LaunchShape*);                                               \
     cudaError_t launch_batch_r##n(const KParams&, int, int, size_t, cudaStream_t, bool);                    \

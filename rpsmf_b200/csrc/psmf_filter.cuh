@@ -21,6 +21,7 @@
 // replicated r x r state never diverges.
 #pragma once
 #include <type_traits>
+#include <cooperative_groups.h>
 #include "psmf_common.cuh"
 
 namespace psmf {
@@ -479,6 +480,10 @@ __device__ __forceinline__ void step_loglik(int flags, double piv, double n, dou
 // instantiation per kernel instead of the GL x LL product.  In the GL-only variant this is a constant, so it compiles as before.
 template <bool GL, bool LL>
 __device__ __forceinline__ bool glin_on(const KParams& p) { return GL && (!LL || (p.flags & F_GRAD_LINEAR) != 0); }
+// The cluster variant (CL) of the direct-load kernel is the LL variant that also serves runs without F_LOGLIK: the 10-wide
+// record and the log-likelihood terms follow the flag.  In every other variant this is the constant LL.
+template <bool LL, bool CL>
+__device__ __forceinline__ bool ll_on(const KParams& p) { return LL && (!CL || (p.flags & F_LOGLIK) != 0); }
 
 // F_GRAD_LINEAR: the accumulator G_A (R * R doubles, row-major) in dynamic shared memory at p.glin_off.  Recomputed where it
 // is used (p lives in the constant bank): no pointer stays live across the row pass.
@@ -707,8 +712,8 @@ __device__ __forceinline__ void lin_grad_step(const KParams& p, Smem<R>& sh, con
 // Gauss-Jordan elimination runs; x, omega, P, Q, rho, lambda follow the elimination.  The arithmetic is the same either
 // way (bit-identical results), only the schedule differs.
 // GL: F_GRAD_LINEAR is set, LL: F_LOGLIK is set (template parameters so that the kernels without them compile to the code they
-// had before them; see glin_on)
-template <int R, int NGJ, bool GL = false, bool LL = false, int BAR = 0, int GJBAR = 1>
+// had before them; see glin_on); CL: the cluster variant, where F_LOGLIK decides at run time (ll_on)
+template <int R, int NGJ, bool GL = false, bool LL = false, int BAR = 0, int GJBAR = 1, bool CL = false>
 __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, int warp, int series, int64_t t,
                              bool writer, int nthr, const double* totv = nullptr) {
     constexpr int NGm = ngram(R);
@@ -831,7 +836,7 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
             sh.sc[0] = omega; sh.sc[4] = sSe; sh.sc[6] = p.beta * omega;
             if (writer) {
                 if (p.scal_out != nullptr) {
-                    double* so = p.scal_out + ((int64_t)series * p.n_steps + t) * (LL ? NSCAL_LL : NSCAL);
+                    double* so = p.scal_out + ((int64_t)series * p.n_steps + t) * (ll_on<LL, CL>(p) ? NSCAL_LL : NSCAL);
                     so[0] = a; so[1] = eta; so[2] = N; so[3] = omega; so[4] = phi; so[5] = sSe; so[6] = lam; so[7] = rho;
                 }
                 if (!(isfinite(N) && isfinite(omega) && isfinite(phi) && isfinite(xn)) || N == 0.0)
@@ -839,7 +844,7 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
             }
         }
         if constexpr (LL) {
-            if (p.scal_out != nullptr) {
+            if (ll_on<LL, CL>(p) && p.scal_out != nullptr) {
                 // S_obs = C_o Pbar C_o' + diag(rho_i + a): log det from the pivots and sum_obs log(rho_i + a), Delta^2 = s over
                 // the observed rows - b'Kb (s also carries w0 q0 of the missing rows; simplified: S_obs^-1 = diag(w_i), b'Kb = 0)
                 const double q0 = tot[NGm + R + 2];
@@ -980,10 +985,36 @@ __device__ __forceinline__ void gpu_exchange(const KParams& p, double* __restric
 //   cps <= 16 : every CTA reads all partials after one grid barrier
 //   cps  > 16 : reduce-scatter / all-gather through L2: CTA c sums entries {c, c + cps, ..} over all CTAs
 //               (coalesced reads of a transposed partial array), a second barrier publishes the totals.
+//   CL        : the CTAs of one series are a thread-block cluster (cps <= 16, one series per cluster): the partials stay in
+//               shared memory and every CTA reads its peers' through distributed shared memory after one cluster barrier
 // sh.part -> sh.tot; ends with a barrier over the `nthr` threads.
-template <int NST, int NSP, int BAR = 0>
+template <int NST, int NSP, int BAR = 0, bool CL = false>
 __device__ __forceinline__ void grid_reduce(const KParams& p, double* __restrict__ part_v, double* __restrict__ tot, int tid,
                                             int lane, int warp, int64_t t, int series, int part, int nthr) {
+    if constexpr (CL) {
+        // parity double buffer [2][NSP] at the end of the dynamic shared memory (cluster_pub_bytes; the static shared memory of
+        // the RHOV variant at r = 16 has no room left): a CTA writes parity t & 1 again at step t + 2, after the barrier of step
+        // t + 1, which every peer reaches only once it has read step t -- one cluster barrier per step is enough
+        extern __shared__ __align__(16) unsigned char psmf_dyn_smem[];
+        unsigned dyn_bytes;
+        asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(dyn_bytes));
+        cooperative_groups::cluster_group cl = cooperative_groups::this_cluster();
+        double* mine = reinterpret_cast<double*>(psmf_dyn_smem + dyn_bytes) - (2 - (t & 1)) * NSP;
+        for (int e = tid; e < NST; e += nthr) mine[e] = part_v[e];
+        stamp(p, t, 3);
+        cl.sync();
+        stamp(p, t, 4);
+        const int cps = p.cps;
+        for (int e = tid; e < NST; e += nthr) {
+            double v[16];                                  // the addition tree of the cps <= 16 path below: the same bits
+#pragma unroll
+            for (int c = 0; c < 16; ++c) v[c] = c < cps ? *cl.map_shared_rank(mine + e, (unsigned)c) : 0.0;
+            tot[e] = (((v[0] + v[1]) + (v[2] + v[3])) + ((v[4] + v[5]) + (v[6] + v[7]))) +
+                     (((v[8] + v[9]) + (v[10] + v[11])) + ((v[12] + v[13]) + (v[14] + v[15])));
+        }
+        sync_n<BAR>(nthr);
+        return;
+    }
     if (p.cps == 1) {
         for (int e = tid; e < NST; e += nthr) tot[e] = part_v[e];
         sync_n<BAR>(nthr);
@@ -1057,7 +1088,9 @@ __device__ __forceinline__ void observe(const KParams& p, const T* __restrict__ 
 // owns them; general fallback (any alignment, any d) and the path for small problems / batched series ----
 // p.phase (caller-driven statistics exchange, one step per launch): 1 = pass + grid reduction, statistics -> p.stats_ext
 // and residuals -> p.e_ext; 2 = r x r update from p.stats_ext (all-reduced by the caller) + the rank-1 update of C.
-template <int R, typename T, bool RHOV = false, bool GL = false, bool LL = false>
+// CL (batched engines): the CTAs of a series form a thread-block cluster of p.cps CTAs and reduce through distributed shared
+// memory; an ordinary launch, no grid barrier.  Instantiated with GL = LL = true: one variant serves every flag.
+template <int R, typename T, bool RHOV = false, bool GL = false, bool LL = false, bool CL = false>
 __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KParams p) {
     // RHOV with LL: one more statistic, sum m log(rho_i + a), inside the padding
     constexpr int NW = V1_WARPS, NSP = RHOV ? nstat_v_pad(R) : nstat_pad(R), NST = RHOV ? nstat_v(R) + (LL ? 1 : 0) : nstat(R);
@@ -1146,7 +1179,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
                     const double rho_i = inb ? __dmul_rn(rscale, rho0[row]) : 1.0;       // R = omega-scale * diag(R0)  (rPSMF.py:134)
                     wi = 1.0 / (rho_i + aa);                                               // rPSMF.py:92,98,32
                     acc.nrho += mi ? rho_i : 0.0;
-                    if constexpr (LL) if (p.scal_out != nullptr) nlog += mi ? log(rho_i + aa) : 0.0;
+                    if constexpr (LL) if (ll_on<LL, CL>(p) && p.scal_out != nullptr) nlog += mi ? log(rho_i + aa) : 0.0;
                 }
                 row_stats<R>(acc, sh, c, ep, inb, mi, yi, wi, w0, e, yh);
 #pragma unroll
@@ -1178,7 +1211,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
                 for (int w = 0; w < NW; ++w) s += red[w * NSP + e2];
                 part_p[e2] = s;
             }
-            grid_reduce<NST, NSP>(p, part_p, tot_p, tid, lane, warp, t, series, part, blockDim.x);
+            grid_reduce<NST, NSP, 0, CL>(p, part_p, tot_p, tid, lane, warp, t, series, part, blockDim.x);
             stamp(p, t, 5);
         }
         if (p.phase == 1) {
@@ -1192,7 +1225,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
             for (int e = tid; e < NST; e += blockDim.x) tot_p[e] = p.stats_ext[e];
             __syncthreads();
         }
-        small_update<R, GJ_THREADS, GL, LL>(p, sh, tid, lane, warp, series, t, writer, blockDim.x, RHOV ? totv : nullptr);
+        small_update<R, GJ_THREADS, GL, LL, 0, 1, CL>(p, sh, tid, lane, warp, series, t, writer, blockDim.x, RHOV ? totv : nullptr);
         stamp(p, t, 6);
     }
 
@@ -1226,6 +1259,8 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
     }
     if constexpr (GL)
         if (writer && glin_on<GL, LL>(p) && p.grad_out != nullptr) lin_grad_writeout<R>(p.grad_out + (int64_t)series * (R * R + R), glin_acc(p), sh.grad, tid, blockDim.x);
+    // a peer may still read this CTA's partials of the last step: nobody leaves before everybody has read
+    if constexpr (CL) cooperative_groups::this_cluster().sync();
 }
 
 }  // namespace psmf

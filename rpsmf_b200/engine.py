@@ -30,6 +30,11 @@ class FilterEngine:
     ``run(want_loglik=True)`` returns ``nll`` (the incremental negative log-likelihood that the gradients differentiate) and
     ``logpred`` (the one-step predictive log-density log p(y_obs,k | y_<k)), each (S, T) float64 (include/psmf_b200.h
     PSMF_LOGLIK).
+
+    ``n_series`` > 1 batches independent series in one launch.  A series runs on one CTA while it fits one (``ctas`` = 0);
+    longer series, or ``ctas`` = c in 2..16, run on a thread-block cluster of c CTAs per series that sums its statistics
+    through distributed shared memory.  That launch is not cooperative: clusters run in waves when there are more than the
+    device holds at once.  ``launch_info()["ctas"]`` reports the CTAs per series.
     """
 
     def __init__(self, d, r, *, n_series=1, dtype=torch.float64, robust=True, simplified=False,

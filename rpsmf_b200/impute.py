@@ -112,8 +112,10 @@ def fit_repeats(Ys, Cs, Xs, Ms, Mmisses, V, Q0, R0, P, lambda0, sig, Iter, Yorig
                 dtype=torch.float64):
     """All repeats of the imputation experiment in ONE batch (the 100-repeat loop of ExperimentImpute/rPSMF.py:194-232 /
     PSMF.py:140-178): repeat k has its own random mask and initial C, X but the same data set, so the repeats are
-    independent series of equal shape -- the resident batch kernel filters them side by side, one CTA each, C in shared
-    memory.  Arguments are lists over the repeats of what ``robust_PSMF`` / ``ProbabilisticSequentialMatrixFactorizer``
+    independent series of equal shape, filtered side by side in one launch: one CTA per repeat while its C fits the shared
+    memory of a CTA (the resident batch kernel) or its residuals do (the direct-load kernel), and above that a
+    thread-block cluster of up to 16 CTAs per repeat, so data sets of some hundred thousand rows run as one batch too.
+    Arguments are lists over the repeats of what ``robust_PSMF`` / ``ProbabilisticSequentialMatrixFactorizer``
     take per call; returns the lists ``(Epred, Efull, RunTime, InsideBars)`` of what they return per call.  ``Xs[k]`` is
     overwritten in place like ``X`` there."""
     S = len(Ys)
@@ -121,7 +123,7 @@ def fit_repeats(Ys, Cs, Xs, Ms, Mmisses, V, Q0, R0, P, lambda0, sig, Iter, Yorig
     r = np.asarray(Cs[0]).shape[1]
     rho0 = _uniform_diag(R0, d, "R")
     if np.ndim(rho0) != 0:
-        raise NotImplementedError("fit_repeats runs on the batch kernel: R must be rho * I (use the per-repeat functions)")
+        raise NotImplementedError("fit_repeats runs as one batched engine: R must be rho * I (use the per-repeat functions)")
     dev = torch.device("cuda", torch.cuda.current_device() if device is None else device)
     t0 = time.time()
     Yt = torch.stack([ingest(Ys[k], dtype=dtype, keep_nan=False, want_mask=False, device=dev.index)[0] for k in range(S)])
