@@ -253,6 +253,37 @@ int  psmf_launch_info2(psmf_handle h, int32_t* kernel, int32_t* nslot, int32_t* 
  * per-CTA pass end / start times; scratch/trace.py decodes them).  dev_buf == NULL disables.           */
 int  psmf_set_trace(psmf_handle h, uint64_t* dev_buf, int32_t steps);
 
+/* per-step moment record of the filter, the input of the fixed-interval smoother below: float64 in both storage types,
+ * PSMF_NMOM(r) doubles per series and step,
+ *   [ x_bar_t (r) | F_t (r x r, row-major) | P_bar_t (r x r) | x_t (r) | P_t (r x r) ]   at the offsets PSMF_MOM_*(r).
+ * x_bar_t, P_bar_t = F_t P_{t-1} F_t' + Q_{t-1} entered step t's update; x_t and P_t left it (P_t as the engine stores it:
+ * beta omega_t (I + P_bar G)^-1 P_bar under PSMF_ROBUST).  F_t is the Jacobian of the predict: I for PSMF_DYN_IDENTITY,
+ * diag(-sin(2 pi theta k + x_{t-1})) for PSMF_DYN_COS, A for PSMF_DYN_LINEAR, F_ext for PSMF_DYN_EXTERNAL.
+ * Every following psmf_run / psmf_run_finish writes the record of its step t (0-based within the call), series s, at
+ * mom + s * series_stride + t * PSMF_NMOM(r); mom == NULL turns it off.  To cover several launches with one horizon, pass a
+ * pointer advanced by the steps already filtered before each launch.  Any kernel, flags (not PSMF_SIMPLIFIED: x_t = x_bar_t
+ * there, PSMF_E_INVALID), dynamics and mask encoding; row-sharded ranks write bit-identical records.  Such runs use the
+ * kernel variant that serves PSMF_LOGLIK; every other output is the same bits as without the record.  series_stride >=
+ * PSMF_NMOM(r) (checked again at each run: >= n_steps * PSMF_NMOM(r)) when n_series > 1.                                   */
+#define PSMF_NMOM(r)       (2 * (r) + 3 * (r) * (r))
+#define PSMF_MOM_XBAR(r)   0
+#define PSMF_MOM_F(r)      (r)
+#define PSMF_MOM_PBAR(r)   ((r) + (r) * (r))
+#define PSMF_MOM_X(r)      ((r) + 2 * (r) * (r))
+#define PSMF_MOM_P(r)      (2 * (r) + 2 * (r) * (r))
+int  psmf_set_moments(psmf_handle h, double* mom, int64_t series_stride);
+
+/* fixed-interval (Rauch-Tung-Striebel) smoother over n_steps records of this engine (psmf_set_moments layout and strides):
+ * x^s_{T-1} = x_{T-1}, P^s_{T-1} = P_{T-1}, and for t = T-2 .. 0
+ *   J_t = P_t F_{t+1}' P_bar_{t+1}^-1,  x^s_t = x_t + J_t (x^s_{t+1} - x_bar_{t+1}),  P^s_t = P_t + J_t (P^s_{t+1} - P_bar_{t+1}) J_t'
+ * -> Xs_out (n_series, n_steps, r) and Ps_out (n_series, n_steps, r, r) or NULL (the r^3 covariance products are then skipped),
+ * contiguous float64.  Conditionally Gaussian given the filter's scales (omega, phi) and linearisation; C is not smoothed.
+ * A singular P_bar_{t+1} (e.g. Q = 0 and P = 0) leaves non-finite rows at t and before.  One CTA per series, gains of a chunk
+ * of steps solved in parallel.  The smoothed reconstruction needs no other kernel: psmf_eval_full(X = Xs) gives Efull of the
+ * smoothed states with the engine's current C, psmf_predict(Xpred_in = Xs) writes C Xs.                                 */
+int  psmf_smooth(psmf_handle h, const double* mom, int64_t series_stride, int64_t n_steps, double* Xs_out, double* Ps_out,
+                 void* stream);
+
 /* multi-GPU row sharding (world_size > 1): NVLink mailbox for the per-step statistics exchange.
  * Each rank exports a blob of PSMF_MAILBOX_BLOB_BYTES (the CUDA IPC handle of its mailbox + a plan record: rank,
  * shape, flags, which kernels its shard is eligible for), gathers all ranks' blobs in rank order through the

@@ -26,12 +26,22 @@ EVAL_SSE, EVAL_INSIDE, EVAL_COUNT = 0, 1, 2
 MAILBOX_BLOB_BYTES = 128
 SCAL_NAMES = ("a", "eta", "N", "omega", "phi", "sSe", "lam", "rho")
 
+
+def NMOM(r):
+    """doubles per series and step of the moment record (psmf_set_moments): [x_bar | F | P_bar | x | P]"""
+    return 2 * r + 3 * r * r
+
+
+def MOM_OFFSETS(r):
+    """offsets of x_bar, F, P_bar, x, P inside one moment record"""
+    return dict(xbar=0, F=r, Pbar=r + r * r, x=r + 2 * r * r, P=2 * r + 2 * r * r)
+
 # every symbol include/psmf_b200.h declares (checked by tests/test_host_cpu.py: the header, this tuple and the built library must agree)
 EXPORTS = (
     "psmf_create", "psmf_destroy", "psmf_last_error", "psmf_version", "psmf_set_state", "psmf_get_state",
     "psmf_run", "psmf_status", "psmf_launch_info", "psmf_launch_info2", "psmf_set_trace", "psmf_mailbox_export", "psmf_mailbox_connect",
     "psmf_stats_buffer", "psmf_run_finish", "psmf_set_linear_dynamics", "psmf_predict", "psmf_eval_full", "psmf_ingest",
-    "psmf_transpose_mask", "psmf_missing_segments", "psmf_count_nan",
+    "psmf_transpose_mask", "psmf_missing_segments", "psmf_count_nan", "psmf_set_moments", "psmf_smooth",
 )
 
 
@@ -99,6 +109,8 @@ def lib():
     L.psmf_transpose_mask.argtypes = [i32, vp, i64, i64, vp, i64, vp]
     L.psmf_missing_segments.argtypes = [i32, i32, vp, i64, vp, i64, i64, i64, vp, i32, vp, vp]
     L.psmf_count_nan.argtypes = [i32, i32, vp, i64, i64, i64, vp, vp]
+    L.psmf_set_moments.argtypes = [vp, vp, i64]
+    L.psmf_smooth.argtypes = [vp, vp, i64, i64, vp, vp, vp]
     for name in EXPORTS:
         if name not in ("psmf_last_error",):
             getattr(L, name).restype = C.c_int

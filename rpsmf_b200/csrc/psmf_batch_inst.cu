@@ -12,10 +12,10 @@ namespace psmf {
 
 template <typename T, int NW>
 static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t st) {
-    // F_LOGLIK: one variant that also serves F_GRAD_LINEAR (glin_on in psmf_filter.cuh)
-    auto kern = (p.flags & F_LOGLIK)        ? psmf_batch_kernel<PSMF_R, T, NW, true, true>
-                : (p.flags & F_GRAD_LINEAR) ? psmf_batch_kernel<PSMF_R, T, NW, true>
-                                            : psmf_batch_kernel<PSMF_R, T, NW>;
+    // F_LOGLIK: one variant that also serves F_GRAD_LINEAR and the moment record (glin_on / ll_on in psmf_filter.cuh)
+    auto kern = ((p.flags & F_LOGLIK) || p.mom) ? psmf_batch_kernel<PSMF_R, T, NW, true, true>
+                : (p.flags & F_GRAD_LINEAR)     ? psmf_batch_kernel<PSMF_R, T, NW, true>
+                                                : psmf_batch_kernel<PSMF_R, T, NW>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     if (e != cudaSuccess) return e;
     kern<<<grid, NW * 32, dyn, st>>>(p);

@@ -9,6 +9,7 @@
 #include "../../include/psmf_b200.h"
 #include "psmf_common.cuh"
 #include "psmf_tools.cuh"
+#include "psmf_smooth.cuh"
 
 PSMF_DECLARE_R(1) PSMF_DECLARE_R(2) PSMF_DECLARE_R(3) PSMF_DECLARE_R(4)
 PSMF_DECLARE_R(5) PSMF_DECLARE_R(6) PSMF_DECLARE_R(7) PSMF_DECLARE_R(8)
@@ -159,6 +160,8 @@ struct psmf_engine {
     size_t tool_bytes = 0;
     unsigned long long* trace = nullptr;
     int trace_steps = 0;
+    double* mom = nullptr;             // psmf_set_moments
+    int64_t mom_sst = 0;
     // NVLink mailbox (world_size > 1): [2 parities][MAX_PEERS][192] tagged 16-byte cells (psmf_filter.cuh gpu_exchange)
     void* mbox = nullptr;
     void* peer_mbox[PSMF_MAX_PEERS] = {nullptr};
@@ -592,6 +595,8 @@ static int run_impl(psmf_handle h, const psmf_io* io, int64_t n_steps, int64_t k
     }
     if (h->cfg.dynamics == PSMF_DYN_LINEAR && !h->lin_set)
         return fail(h, PSMF_E_STATE, "PSMF_DYN_LINEAR: call psmf_set_linear_dynamics first");
+    if (h->mom && h->S > 1 && h->mom_sst < n_steps * nmom(h->R))
+        return fail(h, PSMF_E_INVALID, "psmf_set_moments: series_stride < n_steps * PSMF_NMOM(r), the records of two series would overlap");
     const bool external = h->cfg.exchange == PSMF_XCHG_EXTERNAL;
     if (external) {
         if (n_steps != 1) return fail(h, PSMF_E_INVALID, "PSMF_XCHG_EXTERNAL runs one step per psmf_run / psmf_run_finish pair");
@@ -643,6 +648,7 @@ static int run_impl(psmf_handle h, const psmf_io* io, int64_t n_steps, int64_t k
     }
     p.step_base = h->step_base;       // steps filtered by this engine so far: tags of the mailbox / partial cells
     p.trace = h->trace; p.trace_steps = h->trace_steps;
+    p.mom = h->mom; p.mom_sst = h->mom_sst;
     CK(h, cudaMemsetAsync(h->bar, 0, 8 * sizeof(unsigned long long), st));
     CK(h, cudaMemsetAsync(h->gparams, 0, GPARAMS_BYTES, st));
     if (phase != 2) CK(h, cudaMemsetAsync(h->status, 0xFF, sizeof(long long), st));
@@ -972,6 +978,35 @@ extern "C" int psmf_set_trace(psmf_handle h, uint64_t* dev_buf, int32_t steps) {
     if (!h) return PSMF_E_INVALID;
     h->trace = (unsigned long long*)dev_buf;
     h->trace_steps = dev_buf ? steps : 0;
+    return PSMF_OK;
+}
+
+extern "C" int psmf_set_moments(psmf_handle h, double* mom, int64_t series_stride) {
+    if (!h) return PSMF_E_INVALID;
+    if (mom && (h->cfg.flags & PSMF_SIMPLIFIED))
+        return fail(h, PSMF_E_INVALID, "psmf_set_moments: PSMF_SIMPLIFIED has no filtered covariance to smooth (x_t = x_bar_t)");
+    if (mom && (series_stride < 0 || (h->S > 1 && series_stride < nmom(h->R))))
+        return fail(h, PSMF_E_INVALID, "psmf_set_moments: series_stride must be >= PSMF_NMOM(r) with several series");
+    h->mom = mom;
+    h->mom_sst = mom ? series_stride : 0;
+    return PSMF_OK;
+}
+
+extern "C" int psmf_smooth(psmf_handle h, const double* mom, int64_t series_stride, int64_t n_steps, double* Xs_out, double* Ps_out,
+                           void* stream) {
+    if (!h) return PSMF_E_INVALID;
+    if (!mom || !Xs_out) return fail(h, PSMF_E_INVALID, "psmf_smooth: mom and Xs_out are required");
+    if (h->cfg.flags & PSMF_SIMPLIFIED) return fail(h, PSMF_E_INVALID, "psmf_smooth: a PSMF_SIMPLIFIED engine writes no moment record");
+    if (n_steps < 1) return fail(h, PSMF_E_INVALID, "psmf_smooth: n_steps must be >= 1");
+    if (h->S > 1 && series_stride < n_steps * nmom(h->R))
+        return fail(h, PSMF_E_INVALID, "psmf_smooth: series_stride < n_steps * PSMF_NMOM(r)");
+    CK(h, cudaSetDevice(h->cfg.device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t bytes = smooth_smem_bytes(h->R);
+    CK(h, cudaFuncSetAttribute(smooth_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    smooth_kernel<<<h->S, SM_WARPS * 32, bytes, st>>>(mom, series_stride, n_steps, h->R, Xs_out, Ps_out);
+    CK(h, cudaGetLastError());
+    h->last_stream = st;
     return PSMF_OK;
 }
 

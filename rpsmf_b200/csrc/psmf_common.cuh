@@ -17,6 +17,8 @@ namespace psmf {
 constexpr int TILE = 32;
 constexpr int NSCAL = 8;
 constexpr int NSCAL_LL = 10;   // F_LOGLIK: the record gains [nll_k, log p_k] (include/psmf_b200.h PSMF_SCAL_NLL / PSMF_SCAL_LOGPRED)
+// per-step moment record (include/psmf_b200.h PSMF_NMOM): [x_bar | F (row-major) | P_bar | x | P] float64
+__host__ __device__ constexpr int nmom(int R) { return 2 * R + 3 * R * R; }
 constexpr int MAXR = 16;
 constexpr int MAX_PEERS = 8;
 
@@ -146,6 +148,8 @@ struct KParams {
                               // accumulator G_A (R * R doubles, row-major); the TMA-staged control CTA uses the start
     unsigned long long spin_ns; // a wait (tagged cell, mbarrier, grid barrier, NVLink mailbox) that makes no progress for
                                 // this long gives up: status word <- STATUS_TIMEOUT | step, abort word (bar[7]) <- 1
+    double* mom;              // psmf_set_moments: record of step t, series s at mom + s * mom_sst + t * nmom(R), or nullptr.
+    int64_t mom_sst;          // Written by the LL variant of each kernel only: the launchers pick it when mom is set
 };
 
 // ---- tags and the status word --------------------------------------------------------------------

@@ -480,10 +480,30 @@ __device__ __forceinline__ void step_loglik(int flags, double piv, double n, dou
 // instantiation per kernel instead of the GL x LL product.  In the GL-only variant this is a constant, so it compiles as before.
 template <bool GL, bool LL>
 __device__ __forceinline__ bool glin_on(const KParams& p) { return GL && (!LL || (p.flags & F_GRAD_LINEAR) != 0); }
-// The cluster variant (CL) of the direct-load kernel is the LL variant that also serves runs without F_LOGLIK: the 10-wide
-// record and the log-likelihood terms follow the flag.  In every other variant this is the constant LL.
-template <bool LL, bool CL>
-__device__ __forceinline__ bool ll_on(const KParams& p) { return LL && (!CL || (p.flags & F_LOGLIK) != 0); }
+// The LL variant of each kernel also serves runs without F_LOGLIK: the cluster variant of the direct-load kernel, and every run
+// with a moment record (psmf_set_moments).  The 10-wide record and the log-likelihood terms follow the flag.  In the other
+// variants this is the constant false.
+template <bool LL>
+__device__ __forceinline__ bool ll_on(const KParams& p) { return LL && (p.flags & F_LOGLIK) != 0; }
+
+// psmf_set_moments: entry idx (< R * R) of the moment record of step t, written by the thread that replaces P[idx] with pn.  x_bar,
+// P_bar and F of the step are still in shared memory (the next predict follows) and x already holds x_t.  F is the Jacobian the
+// predict used: diag(fd) for identity (fd = 1) and cos dynamics, A for linear, F_ext for external dynamics.
+template <int R>
+__device__ __forceinline__ void moment_store(const KParams& p, const Smem<R>& sh, int series, int64_t t, int idx, double pn) {
+    double* m = p.mom + (int64_t)series * p.mom_sst + t * nmom(R);
+    const int i = idx / R, j = idx % R;
+    const double f = p.dynamics == DYN_LINEAR     ? p.lin_A[idx]
+                   : p.dynamics == DYN_EXTERNAL ? p.F_ext[(int64_t)series * R * R + idx]
+                                                 : (i == j ? sh.fd[i] : 0.0);
+    m[R + idx] = f;
+    m[R + R * R + idx] = sh.Pb[idx];
+    m[2 * R + 2 * R * R + idx] = pn;
+    if (idx < R) {
+        m[idx] = sh.xb[idx];
+        m[R + 2 * R * R + idx] = sh.x[idx];
+    }
+}
 
 // F_GRAD_LINEAR: the accumulator G_A (R * R doubles, row-major) in dynamic shared memory at p.glin_off.  Recomputed where it
 // is used (p lives in the constant bank): no pointer stays live across the row pass.
@@ -711,8 +731,8 @@ __device__ __forceinline__ void lin_grad_step(const KParams& p, Smem<R>& sh, con
 // when the CTA has a warp outside the NGJ elimination threads (nthr >= NGJ + 32) that warp computes them WHILE the
 // Gauss-Jordan elimination runs; x, omega, P, Q, rho, lambda follow the elimination.  The arithmetic is the same either
 // way (bit-identical results), only the schedule differs.
-// GL: F_GRAD_LINEAR is set, LL: F_LOGLIK is set (template parameters so that the kernels without them compile to the code they
-// had before them; see glin_on); CL: the cluster variant, where F_LOGLIK decides at run time (ll_on)
+// GL: F_GRAD_LINEAR may be set, LL: F_LOGLIK or a moment record may be set (template parameters so that the kernels without them
+// compile to the code they had before them; see glin_on / ll_on); CL: the cluster variant
 template <int R, int NGJ, bool GL = false, bool LL = false, int BAR = 0, int GJBAR = 1, bool CL = false>
 __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, int warp, int series, int64_t t,
                              bool writer, int nthr, const double* totv = nullptr) {
@@ -836,7 +856,7 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
             sh.sc[0] = omega; sh.sc[4] = sSe; sh.sc[6] = p.beta * omega;
             if (writer) {
                 if (p.scal_out != nullptr) {
-                    double* so = p.scal_out + ((int64_t)series * p.n_steps + t) * (ll_on<LL, CL>(p) ? NSCAL_LL : NSCAL);
+                    double* so = p.scal_out + ((int64_t)series * p.n_steps + t) * (ll_on<LL>(p) ? NSCAL_LL : NSCAL);
                     so[0] = a; so[1] = eta; so[2] = N; so[3] = omega; so[4] = phi; so[5] = sSe; so[6] = lam; so[7] = rho;
                 }
                 if (!(isfinite(N) && isfinite(omega) && isfinite(phi) && isfinite(xn)) || N == 0.0)
@@ -844,7 +864,7 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
             }
         }
         if constexpr (LL) {
-            if (ll_on<LL, CL>(p) && p.scal_out != nullptr) {
+            if (ll_on<LL>(p) && p.scal_out != nullptr) {
                 // S_obs = C_o Pbar C_o' + diag(rho_i + a): log det from the pivots and sum_obs log(rho_i + a), Delta^2 = s over
                 // the observed rows - b'Kb (s also carries w0 q0 of the missing rows; simplified: S_obs^-1 = diag(w_i), b'Kb = 0)
                 const double q0 = tot[NGm + R + 2];
@@ -865,7 +885,9 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
         const double omega = sh.sc[0], bom = sh.sc[6];
         for (int idx = tid; idx < R * R; idx += nthr) {
             const int i = idx / R, j = idx % R;
-            sh.P[idx] = simp ? sh.Pb[idx] : bom * sh.aug[FIN][sh.perm[i]][R + j];          // rPSMF.py:106
+            const double pn = simp ? sh.Pb[idx] : bom * sh.aug[FIN][sh.perm[i]][R + j];     // rPSMF.py:106
+            if constexpr (LL) if (writer && p.mom != nullptr) moment_store<R>(p, sh, series, t, idx, pn);
+            sh.P[idx] = pn;
             if (!simp) sh.Q[idx] = omega * sh.Q[idx];                                        // rPSMF.py:133
         }
         if (tid == nthr - 32) {
@@ -1179,7 +1201,7 @@ __global__ void __launch_bounds__(V1_WARPS * 32, 2) psmf_filter_kernel(const KPa
                     const double rho_i = inb ? __dmul_rn(rscale, rho0[row]) : 1.0;       // R = omega-scale * diag(R0)  (rPSMF.py:134)
                     wi = 1.0 / (rho_i + aa);                                               // rPSMF.py:92,98,32
                     acc.nrho += mi ? rho_i : 0.0;
-                    if constexpr (LL) if (ll_on<LL, CL>(p) && p.scal_out != nullptr) nlog += mi ? log(rho_i + aa) : 0.0;
+                    if constexpr (LL) if (ll_on<LL>(p) && p.scal_out != nullptr) nlog += mi ? log(rho_i + aa) : 0.0;
                 }
                 row_stats<R>(acc, sh, c, ep, inb, mi, yi, wi, w0, e, yh);
 #pragma unroll

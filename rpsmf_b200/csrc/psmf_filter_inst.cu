@@ -13,10 +13,10 @@ namespace psmf {
 
 template <typename T, bool RHOV = false>
 static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t st, bool coop) {
-    // F_LOGLIK: one variant that also serves F_GRAD_LINEAR (glin_on in psmf_filter.cuh)
-    auto kern = (p.flags & F_LOGLIK)        ? psmf_filter_kernel<PSMF_R, T, RHOV, true, true>
-                : (p.flags & F_GRAD_LINEAR) ? psmf_filter_kernel<PSMF_R, T, RHOV, true>
-                                            : psmf_filter_kernel<PSMF_R, T, RHOV>;
+    // F_LOGLIK: one variant that also serves F_GRAD_LINEAR and the moment record (glin_on / ll_on in psmf_filter.cuh)
+    auto kern = ((p.flags & F_LOGLIK) || p.mom) ? psmf_filter_kernel<PSMF_R, T, RHOV, true, true>
+                : (p.flags & F_GRAD_LINEAR)     ? psmf_filter_kernel<PSMF_R, T, RHOV, true>
+                                                : psmf_filter_kernel<PSMF_R, T, RHOV>;
     constexpr int threads = V1_WARPS * 32;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     if (e != cudaSuccess) return e;

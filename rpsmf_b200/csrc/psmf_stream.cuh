@@ -923,14 +923,14 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
                 sh.sc[0] = omega; sh.sc[3] = phi; sh.sc[4] = sSe;
                 sh.sc[5] = p.alpha * phi; sh.sc[6] = p.beta * omega;
                 if (p.scal_out != nullptr) {
-                    double* so = p.scal_out + t * (LL ? NSCAL_LL : NSCAL);
+                    double* so = p.scal_out + t * (ll_on<LL>(p) ? NSCAL_LL : NSCAL);
                     so[0] = a; so[1] = eta; so[2] = N; so[3] = omega; so[4] = phi; so[5] = sSe; so[6] = lam; so[7] = rho;
                 }
                 if (!(isfinite(N) && isfinite(omega) && isfinite(phi) && isfinite(xn)) || N == 0.0)
                     atomicCAS((unsigned long long*)p.status, ~0ULL, (unsigned long long)t);
             }
             if constexpr (LL) {
-                if (p.scal_out != nullptr) {           // as in small_update (psmf_filter.cuh), uniform R
+                if (ll_on<LL>(p) && p.scal_out != nullptr) {   // as in small_update (psmf_filter.cuh), uniform R
                     const double piv = (!simp && lane < R) ? sh.aug[0][lane][2 * R + 1] : 1.0;
                     double nll, lp;
                     step_loglik(p.flags, piv, nobs, N, q1, lam, nobs * log(rho + a), sh.w1 * q1 - bkb, lane, nll, lp);
@@ -949,6 +949,7 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
                 const int i = idx / R, j = idx % R;
                 const double pn = simp ? sh.Pb[idx] : bom * sh.aug[FIN][sh.perm[i]][R + j];      // rPSMF.py:106
                 const double vn = aphi * (sh.V[idx] - sh.vx[i] * sh.vxt[j] / N);                 // rPSMF.py:115
+                if constexpr (LL) if (p.mom != nullptr) moment_store<R>(p, sh, 0, t, idx, pn);
                 sh.P[idx] = pn;
                 sh.V[idx] = vn;
                 if (!simp) sh.Q[idx] = omega * sh.Q[idx];                                        // rPSMF.py:133

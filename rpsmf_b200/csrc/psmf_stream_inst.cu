@@ -12,10 +12,10 @@ namespace psmf {
 
 template <typename T>
 static cudaError_t launch_t(const KParams& p, int grid, size_t dyn, cudaStream_t st, bool coop) {
-    // F_LOGLIK: one variant that also serves F_GRAD_LINEAR (glin_on in psmf_filter.cuh)
-    auto kern = (p.flags & F_LOGLIK)        ? psmf_stream_kernel<PSMF_R, T, true, true>
-                : (p.flags & F_GRAD_LINEAR) ? psmf_stream_kernel<PSMF_R, T, true>
-                                            : psmf_stream_kernel<PSMF_R, T>;
+    // F_LOGLIK: one variant that also serves F_GRAD_LINEAR and the moment record (glin_on / ll_on in psmf_filter.cuh)
+    auto kern = ((p.flags & F_LOGLIK) || p.mom) ? psmf_stream_kernel<PSMF_R, T, true, true>
+                : (p.flags & F_GRAD_LINEAR)     ? psmf_stream_kernel<PSMF_R, T, true>
+                                                : psmf_stream_kernel<PSMF_R, T>;
     constexpr int threads = s_threads();
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn);
     if (e != cudaSuccess) return e;

@@ -35,6 +35,10 @@ class FilterEngine:
     longer series, or ``ctas`` = c in 2..16, run on a thread-block cluster of c CTAs per series that sums its statistics
     through distributed shared memory.  That launch is not cooperative: clusters run in waves when there are more than the
     device holds at once.  ``launch_info()["ctas"]`` reports the CTAs per series.
+
+    Smoothing: ``run(want_moments=True)`` (or ``moments_out``) returns the per-step moment record ``moments`` (S, T, NMOM(r))
+    float64 (include/psmf_b200.h psmf_set_moments), and ``smooth(moments)`` runs the fixed-interval (RTS) smoother over it on
+    the device.
     """
 
     def __init__(self, d, r, *, n_series=1, dtype=torch.float64, robust=True, simplified=False,
@@ -145,7 +149,7 @@ class FilterEngine:
     # -- the hot path ------------------------------------------------------------------------------
     def run(self, Y, M=None, k0=1, want_X=True, want_Yrec=False, want_scal=False, xbar=None, F=None,
             X_out=None, Yrec_out=None, scal_out=None, want_grad=False, Yorig=None, E=None, sig=2.0, want_loglik=False,
-            _finish=False):
+            want_moments=False, moments_out=None, _finish=False):
         """Filter ``T`` steps.  Y: device tensor (T, d) or (S, T, d) in the engine dtype (last dim may be
         padded: ld = stride of the time axis); M: uint8 tensor of the same shape or None.
 
@@ -154,7 +158,11 @@ class FilterEngine:
         run: [sum (y_hat - y_orig)^2, entries inside y_hat -+ sig sqrt(U), entries of E, 0].
 
         ``want_loglik`` (an engine created with ``loglik=True``): ``nll`` and ``logpred``, (S, T) views of the 10-wide scalar
-        record, which ``scal`` then is."""
+        record, which ``scal`` then is.
+
+        ``want_moments`` / ``moments_out``: ``moments`` = (S, T, NMOM(r)) float64 record [x_bar | F | P_bar | x | P] of every
+        step, the input of ``smooth``.  ``moments_out`` may be a view into a longer horizon (S, T_total, NMOM(r)) advanced by
+        the steps already filtered; its series stride is kept.  The record is set for this launch only."""
         S, d, r = self.S, self.d, self.r
         if not isinstance(Y, torch.Tensor) or Y.device != self.device:
             raise ValueError("Y must be a tensor on %s" % self.device)
@@ -231,11 +239,28 @@ class FilterEngine:
                 Ft = _dev_tensor(F, torch.float64, self.device).reshape(S, r, r)
                 io.F_ext = Ft.data_ptr()
                 keep.append(Ft)
+        mom = None
+        if want_moments or moments_out is not None:
+            nm = _capi.NMOM(r)
+            mom = moments_out if moments_out is not None else torch.empty((S, T, nm), dtype=torch.float64, device=self.device)
+            if mom.dim() == 2:
+                mom = mom.unsqueeze(0)
+            if (mom.dtype != torch.float64 or mom.device != self.device or tuple(mom.shape) != (S, T, nm) or mom.stride(2) != 1
+                    or mom.stride(1) != nm):
+                raise ValueError("moments_out must be a float64 (S, T, %d) tensor on %s, contiguous per series" % (nm, self.device))
+            res["moments"] = mom
+            keep.append(mom)
         with torch.cuda.device(self.device):
-            if _finish:
-                self._ck(self._L.psmf_run_finish(self._h, C.byref(io), int(k0), self._stream()))
-            else:
-                self._ck(self._L.psmf_run(self._h, C.byref(io), T, int(k0), self._stream()))
+            if mom is not None:
+                self._ck(self._L.psmf_set_moments(self._h, C.c_void_p(mom.data_ptr()), mom.stride(0)))
+            try:
+                if _finish:
+                    self._ck(self._L.psmf_run_finish(self._h, C.byref(io), int(k0), self._stream()))
+                else:
+                    self._ck(self._L.psmf_run(self._h, C.byref(io), T, int(k0), self._stream()))
+            finally:
+                if mom is not None:
+                    self._L.psmf_set_moments(self._h, None, 0)
         self._keep_run = keep
         if S == 1:
             res = {k: v[0] for k, v in res.items()}
@@ -378,6 +403,29 @@ class FilterEngine:
                                             C.c_void_p(out.data_ptr()), self._stream()))
         self._keep_eval = (X, Yorig, E)
         return out
+
+    def smooth(self, moments, want_P=False, check=True):
+        """Fixed-interval (Rauch-Tung-Striebel) smoother over the moment record of ``run(want_moments=True)`` (S, T, NMOM(r)),
+        one horizon of T steps, possibly written by several launches: returns Xs (S, T, r), and with ``want_P`` also Ps
+        (S, T, r, r), float64 on the device.  Raises FloatingPointError on a non-finite result (a singular P_bar); with
+        ``check=False`` the non-finite rows are returned as they are, for the caller to mask per series."""
+        S, r = self.S, self.r
+        nm = _capi.NMOM(r)
+        mom = moments.unsqueeze(0) if moments.dim() == 2 else moments
+        if (mom.dtype != torch.float64 or mom.device != self.device or mom.dim() != 3 or mom.shape[0] != S or mom.shape[2] != nm
+                or mom.stride(2) != 1 or mom.stride(1) != nm):
+            raise ValueError("moments must be a float64 (S, T, %d) tensor on %s, contiguous per series" % (nm, self.device))
+        T = mom.shape[1]
+        Xs = torch.empty((S, T, r), dtype=torch.float64, device=self.device)
+        Ps = torch.empty((S, T, r, r), dtype=torch.float64, device=self.device) if want_P else None
+        with torch.cuda.device(self.device):
+            self._ck(self._L.psmf_smooth(self._h, C.c_void_p(mom.data_ptr()), mom.stride(0), T, C.c_void_p(Xs.data_ptr()),
+                                         None if Ps is None else C.c_void_p(Ps.data_ptr()), self._stream()))
+        if check and (not bool(torch.isfinite(Xs).all()) or (Ps is not None and not bool(torch.isfinite(Ps).all()))):
+            raise FloatingPointError("smoother: non-finite smoothed moments (singular predicted covariance P_bar)")
+        if S == 1:
+            Xs, Ps = Xs[0], (None if Ps is None else Ps[0])
+        return (Xs, Ps) if want_P else Xs
 
     def connect(self, dist):
         """Row sharding over several GPUs: exchange the mailbox blobs (CUDA IPC handle + plan record) through the

@@ -29,6 +29,10 @@ What differs, by design:
   negative log-likelihood whose gradient the optimisers descend, and ``_logpred[i]`` = sum_k log p(y_k | y_<k), the
   one-step predictive log-likelihood, both computed in the filter kernel (include/psmf_b200.h PSMF_LOGLIK).  The Recursive
   variants make one sweep: key 1, summed over their ``update_every`` blocks.
+* ``smooth=True`` (keyword-only, all classes): after each sweep, ``_mu_smooth[k]`` (r, 1) and ``_P_smooth[k]`` (r, r), k = 1..T,
+  hold the fixed-interval (Rauch-Tung-Striebel) smoothed states of that sweep: every launch of the sweep writes its per-step
+  moment record into one horizon on the device and ``FilterEngine.smooth`` runs the backward pass there.  Not with
+  ``simplified=True`` (x_t = x_bar_t has no filtered covariance to smooth).
 """
 
 from __future__ import annotations
@@ -83,7 +87,9 @@ class PSMFIter:
     _ll_student = False
 
     def __init__(self, theta0, C0, V0, mu0, P0, Qs, Rs, nonlinearity, optim="adam", simplified=False, device=None,
-                 dtype=torch.float64, *, loglik=False):
+                 dtype=torch.float64, *, loglik=False, smooth=False):
+        if smooth and simplified:
+            raise ValueError("smooth=True needs the full filter: simplified=True keeps no filtered covariance (x_t = x_bar_t)")
         self.nonlinearity = nonlinearity
         assert optim in ["adam", "sgd"]
         self.optim = optim
@@ -122,6 +128,10 @@ class PSMFIter:
         self._objective = {}
         self._logpred = {}
         self._llsum = None
+        self._smooth = bool(smooth)
+        self._mu_smooth = {}
+        self._P_smooth = {}
+        self._mom = None
 
     # ---- configuration handed to the kernel ----------------------------------------------------------
     def _q_rho(self):
@@ -222,14 +232,20 @@ class PSMFIter:
             self._yrec_from = k_first
         if getattr(self, "_yrec_from", None) is None:
             self._yrec_from = k_first
+        # smooth: the moment records of every launch of the sweep go into one (1, T, NMOM) horizon on the device
+        mom = None
+        if self._smooth:
+            if self._mom is None or self._mom.shape[1] != T_all or self._mom.device != Yd.device:
+                self._mom = torch.empty((1, T_all, _capi.NMOM(self._r)), dtype=torch.float64, device=Yd.device)
+            mom = self._mom[:, k_first - 1:k_last]
         if self._dyn == _capi.DYN_EXTERNAL:
-            buf[k_first - 1:k_last] = self._sweep_external(eng, ysl, msl, theta, k_first, n)     # accumulates self._gradsum itself
+            buf[k_first - 1:k_last] = self._sweep_external(eng, ysl, msl, theta, k_first, n, mom)   # accumulates self._gradsum itself
             grad = None
         elif self._dyn == _capi.DYN_LINEAR:
             eng.set_linear_dynamics(*self.nonlinearity.parts(theta, self._r))
             learn = np.asarray(theta).size > 0
             out = eng.run(ysl, msl, k0=k_first, want_X=False, Yrec_out=buf[k_first - 1:k_last].unsqueeze(0), want_grad=learn,
-                          want_loglik=self._loglik)
+                          want_loglik=self._loglik, moments_out=mom)
             self._add_loglik(out)
             grad = None
             if learn:
@@ -239,7 +255,7 @@ class PSMFIter:
                 self._gradsum = self._gradsum + g.reshape(self._gradsum.shape)
         else:
             out = eng.run(ysl, msl, k0=k_first, want_X=False, Yrec_out=buf[k_first - 1:k_last].unsqueeze(0),
-                          want_grad=self._dyn == _capi.DYN_COS, want_loglik=self._loglik)
+                          want_grad=self._dyn == _capi.DYN_COS, want_loglik=self._loglik, moments_out=mom)
             self._add_loglik(out)
             grad = out.get("grad")
         bad = eng.status()
@@ -264,9 +280,14 @@ class PSMFIter:
         self._mu = {k_last: st["x"].cpu().numpy().reshape(self._r, 1)}
         self._P = {k_last: st["P"].cpu().numpy()}
         self._V = {k_last: st["V"].cpu().numpy()}
+        if self._smooth:
+            Xs, Ps = eng.smooth(self._mom[:, :k_last], want_P=True)
+            Xs, Ps = Xs.cpu().numpy(), Ps.cpu().numpy()
+            self._mu_smooth = {k: Xs[k - 1].reshape(self._r, 1) for k in range(1, k_last + 1)}
+            self._P_smooth = {k: Ps[k - 1] for k in range(1, k_last + 1)}
         self._after_sweep(st, k_last)
 
-    def _sweep_external(self, eng, ysl, msl, theta, k_first, n):
+    def _sweep_external(self, eng, ysl, msl, theta, k_first, n, mom=None):
         """Arbitrary callable dynamics: x_bar and F = df/dx from the host, one step per launch."""
         Yrec = torch.empty((n, self._d), dtype=self._dtype, device=eng.device)
         learn = np.asarray(theta).size > 0
@@ -276,7 +297,8 @@ class PSMFIter:
             xbar = np.asarray(self.nonlinearity(theta, x, k), dtype=np.float64).reshape(self._r)
             F = None if self._simplified else jacobian_x(self.nonlinearity, theta, x, k)
             out = eng.run(ysl[j:j + 1], None if msl is None else msl[j:j + 1], k0=k, want_X=False, Yrec_out=Yrec[j:j + 1],
-                          xbar=xbar, F=F, want_grad=learn, want_loglik=self._loglik)
+                          xbar=xbar, F=F, want_grad=learn, want_loglik=self._loglik,
+                          moments_out=None if mom is None else mom[:, j:j + 1])
             self._add_loglik(out)
             if learn:
                 # d ell_k / d theta = J_theta' d ell_k / d f  (psmf.py:167-177): the kernel returns d ell_k / d f

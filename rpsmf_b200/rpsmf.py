@@ -18,10 +18,10 @@ class rPSMFIter(PSMFIter):
     _ll_student = True
 
     def __init__(self, theta0, C0, V0, mu0, P0, Q0, R0, lambda0, nonlinearity, fixed_lambda=False, use_scaling=False,
-                 optim="adam", simplified=False, device=None, dtype=torch.float64, *, loglik=False):
+                 optim="adam", simplified=False, device=None, dtype=torch.float64, *, loglik=False, smooth=False):
         assert optim in ["adam", "sgd"]
         super().__init__(theta0, C0, V0, mu0, P0, Q0, R0, nonlinearity, optim=optim, simplified=simplified,
-                         device=device, dtype=dtype, loglik=loglik)
+                         device=device, dtype=dtype, loglik=loglik, smooth=smooth)
         self.Q0 = Q0
         self.R0 = R0
         self.lambda0 = lambda0
