@@ -235,7 +235,9 @@ int  psmf_missing_segments(int32_t device, int32_t dtype, void* Y, int64_t ldy, 
 int  psmf_count_nan(int32_t device, int32_t dtype, const void* Y, int64_t ldy, int64_t d, int64_t n, uint64_t* count_dev, void* stream);
 
 /* synchronise the stream of the last run and report the device status word:
- * *first_bad_step = -1 if every step produced finite N/omega/phi, else the first offending step.
+ * *first_bad_step = -1 if every step of the last run produced finite N/omega/phi/x with N != 0, else the smallest step
+ * (0-based within that run, over all series of the engine) at which any series did not, whatever order the series ran in.
+ * Every psmf_run starts the report afresh; psmf_run_finish completes the step of the psmf_run before it.
  * Returns PSMF_E_STATE (text in psmf_last_error) if a wait inside the kernel expired -- a peer GPU or CTA stopped
  * answering for PSMF_SPIN_TIMEOUT_MS (environment, default 10000) -- or if a peer GPU turned out to run a
  * different kernel; the launch has then drained with invalid results instead of hanging.              */

@@ -485,8 +485,8 @@ extern "C" int psmf_create(psmf_handle* out, const psmf_config* cfg) {
     }
     CKC(cudaMalloc(&e->bar, 8 * sizeof(unsigned long long)));
     CKC(cudaMalloc(&e->gparams, GPARAMS_BYTES));                        // 16-byte cells (psmf_stream.cuh): parameter sets [2][2R], totals [2][nstat2_pad]
-    CKC(cudaMalloc(&e->status, sizeof(long long)));
-    CKC(cudaMemset(e->status, 0xFF, sizeof(long long)));
+    CKC(cudaMalloc(&e->status, STATUS_WORDS * sizeof(long long)));
+    CKC(cudaMemset(e->status, 0xFF, STATUS_WORDS * sizeof(long long)));
     if (cfg->world_size > 1 && cfg->exchange == PSMF_XCHG_NVLINK) {
         CKC(cudaMalloc(&e->mbox, mbox_bytes()));
         CKC(cudaMemset(e->mbox, 0, mbox_bytes()));
@@ -651,7 +651,7 @@ static int run_impl(psmf_handle h, const psmf_io* io, int64_t n_steps, int64_t k
     p.mom = h->mom; p.mom_sst = h->mom_sst;
     CK(h, cudaMemsetAsync(h->bar, 0, 8 * sizeof(unsigned long long), st));
     CK(h, cudaMemsetAsync(h->gparams, 0, GPARAMS_BYTES, st));
-    if (phase != 2) CK(h, cudaMemsetAsync(h->status, 0xFF, sizeof(long long), st));
+    if (phase != 2) CK(h, cudaMemsetAsync(h->status, 0xFF, STATUS_WORDS * sizeof(long long), st));
     // ---- which kernel ----
     // the resident batch kernel: independent series / one small series, C in shared memory for the whole launch
     bool use3 = h->batch_ok && !external &&
@@ -935,8 +935,9 @@ extern "C" int psmf_status(psmf_handle h, int64_t* first_bad_step) {
     if (!h) return PSMF_E_INVALID;
     CK(h, cudaSetDevice(h->cfg.device));
     CK(h, cudaStreamSynchronize(h->last_stream));
-    long long v = -1;
-    CK(h, cudaMemcpy(&v, h->status, sizeof(v), cudaMemcpyDeviceToHost));
+    long long w[STATUS_WORDS];
+    CK(h, cudaMemcpy(w, h->status, sizeof(w), cudaMemcpyDeviceToHost));
+    const long long v = w[0];
     if (v >= 0 && (v & (STATUS_TIMEOUT | STATUS_MISMATCH)) != 0) {
         const long long step = v & 0xFFFFFFFFFFFFLL;
         if (first_bad_step) *first_bad_step = (int64_t)step;
@@ -952,7 +953,7 @@ extern "C" int psmf_status(psmf_handle h, int64_t* first_bad_step) {
         return fail(h, PSMF_E_STATE, "a peer GPU runs a different kernel / statistics layout (mailbox header mismatch at step " +
                                          std::to_string(step) + ")");
     }
-    if (first_bad_step) *first_bad_step = (int64_t)v;
+    if (first_bad_step) *first_bad_step = (int64_t)w[1];
     return PSMF_OK;
 }
 

@@ -111,7 +111,7 @@ struct KParams {
     double* grad_out;         // (n_series, R) accumulated theta gradient, F_GRAD_LINEAR: (n_series, R*R + R) [G_A | G_c]; or nullptr
     double* partials;         // direct kernel: grid_reduce scratch; pipelined kernel: [2][nstat2_pad][pstr] tagged cells
     unsigned long long* bar;  // direct kernel: grid barrier counter; pipelined kernel: [0..1] arrival counters, [2] flag
-    long long* status;        // first bad step or -1
+    long long* status;        // [0] timeout / mismatch code, [1] first bad step; -1 = none
     int64_t d, d_global;
     int64_t n_steps, k0;
     int32_t n_series, cps;    // CTAs per series
@@ -156,10 +156,18 @@ struct KParams {
 // Tags of the 16-byte cells: never 0 (zeroed memory must not look valid), period 2^31 steps.  A stale cell holds
 // the tag of two steps earlier (two parities), so a wrapped tag can never be mistaken for a current one.
 __host__ __device__ constexpr uint32_t tag_of(unsigned long long step) { return (uint32_t)step | 0x80000000u; }
-// status word (KParams.status, int64): -1 = ok, >= 0 = first step with a non-finite N / omega / phi / x,
-// STATUS_TIMEOUT | (where << 48) | step = a bounded wait expired (peer GPU or CTA gone): psmf_status -> PSMF_E_STATE
+// status words (KParams.status, int64[2]), both reset to -1 (all bits set) by every launch:
+//   [0] STATUS_TIMEOUT | (where << 48) | step = a bounded wait expired (peer GPU or CTA gone): psmf_status -> PSMF_E_STATE;
+//       STATUS_MISMATCH | step = a peer runs another kernel / statistics layout (mailbox header)
+//   [1] smallest step (launch-relative, over every series) with a non-finite N / omega / phi / x or N == 0, else -1
 constexpr long long STATUS_TIMEOUT = 1LL << 62;
-constexpr long long STATUS_MISMATCH = 1LL << 61;     // peer runs another kernel / statistics layout (mailbox header)
+constexpr long long STATUS_MISMATCH = 1LL << 61;
+constexpr int STATUS_WORDS = 2;
+// An unsigned minimum over the empty word ~0: the earliest bad step wins whatever order the series ran in (a batched engine
+// runs its series in waves when they outnumber the device), and a timeout or mismatch in word 0 is never overwritten.
+__device__ __forceinline__ void status_bad_step(long long* status, long long t) {
+    atomicMin((unsigned long long*)status + 1, (unsigned long long)t);
+}
 constexpr int ABORT_WORD = 7;                          // index into KParams.bar
 enum SpinSite { SPIN_CELL = 1, SPIN_PEER = 2, SPIN_MBAR = 3, SPIN_GRID = 4, SPIN_RING = 5, SPIN_PARTIALS = 6 };
 // NVLink mailbox: [2 parities][MAX_PEERS] slots of MBOX_SLOT tagged cells; the last cell of a slot is the header

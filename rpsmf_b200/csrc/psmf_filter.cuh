@@ -860,7 +860,7 @@ __device__ void small_update(const KParams& p, Smem<R>& sh, int tid, int lane, i
                     so[0] = a; so[1] = eta; so[2] = N; so[3] = omega; so[4] = phi; so[5] = sSe; so[6] = lam; so[7] = rho;
                 }
                 if (!(isfinite(N) && isfinite(omega) && isfinite(phi) && isfinite(xn)) || N == 0.0)
-                    atomicCAS((unsigned long long*)p.status, ~0ULL, (unsigned long long)t);
+                    status_bad_step(p.status, t);
             }
         }
         if constexpr (LL) {

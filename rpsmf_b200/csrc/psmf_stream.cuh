@@ -927,7 +927,7 @@ __device__ void control_solve(const KParams& p, ControlSmem<R>& cs) {
                     so[0] = a; so[1] = eta; so[2] = N; so[3] = omega; so[4] = phi; so[5] = sSe; so[6] = lam; so[7] = rho;
                 }
                 if (!(isfinite(N) && isfinite(omega) && isfinite(phi) && isfinite(xn)) || N == 0.0)
-                    atomicCAS((unsigned long long*)p.status, ~0ULL, (unsigned long long)t);
+                    status_bad_step(p.status, t);
             }
             if constexpr (LL) {
                 if (ll_on<LL>(p) && p.scal_out != nullptr) {   // as in small_update (psmf_filter.cuh), uniform R

@@ -270,7 +270,7 @@ class FilterEngine:
         """Filter a long HOST-resident sequence: Y_host (T, d) pinned CPU tensor in the engine dtype, M_host
         (T, d) uint8.  Windows of ``window`` steps are copied host->device on a side stream while the
         previous window is being filtered (double buffering); returns X (T, r) on the host (pinned).
-        Single-series engines only."""
+        Single-series engines only.  Each window is one launch, so ``status()`` afterwards describes the last window only."""
         if self.S != 1:
             raise ValueError("run_host supports single-series engines")
         T, d = Y_host.shape[0], self.d
@@ -446,7 +446,9 @@ class FilterEngine:
         dist.barrier()
 
     def status(self):
-        """Synchronise and return the first step with a non-finite N/omega/phi/x, or -1."""
+        """Synchronise and return the smallest step of the last launch, counted from 0 within that launch and taken over
+        every series of the engine, at which a series produced a non-finite N/omega/phi/x or N == 0; -1 if there was none.
+        Every launch starts the report afresh."""
         bad = C.c_int64(-1)
         self._ck(self._L.psmf_status(self._h, C.byref(bad)))
         return int(bad.value)

@@ -299,6 +299,9 @@ class PSMFIter:
             out = eng.run(ysl[j:j + 1], None if msl is None else msl[j:j + 1], k0=k, want_X=False, Yrec_out=Yrec[j:j + 1],
                           xbar=xbar, F=F, want_grad=learn, want_loglik=self._loglik,
                           moments_out=None if mom is None else mom[:, j:j + 1])
+            # every launch resets the status word: check each step before its state reaches the callable
+            if eng.status() >= 0:
+                raise FloatingPointError("non-finite filter state at step %d" % k)
             self._add_loglik(out)
             if learn:
                 # d ell_k / d theta = J_theta' d ell_k / d f  (psmf.py:167-177): the kernel returns d ell_k / d f
